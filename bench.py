@@ -2,6 +2,7 @@
 """bench.py — the headline benchmark of BASELINE.json on B200.
 
   python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C2|C1|C3|C4|C4f32|C4f64|C5|S1|S2|T1]
+                  [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] — causal_1d fp16 forward + backward,
 batch x heads = 16 x 16, head_dim 128, seq 8192 (GPT-style self-attention), inputs U(-2,2) already
@@ -18,6 +19,7 @@ The product path is libfa_b200.so through its C ABI (ctypes); torch only owns de
 streams and the process group. oracle/ is used solely for the cpu_baseline / --impl reference legs.
 """
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
@@ -107,6 +109,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "20"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.terminate)     # the sampler never outlives a run that fails before stop()
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -166,6 +169,28 @@ def flops_of(w, nnz):
     return 2.0 * nnz * (w["d"] + w["v_d"]) * b, 2.0 * nnz * (3 * w["d"] + 2 * w["v_d"]) * b
 
 
+DUMP_BYTES = 64 * 10 ** 6   # --dump-outputs writes at most this many bytes in all, .npy headers included
+
+
+def dump_outputs(out_dir, outputs, rank, world):
+    """Writes each device tensor of `outputs` (name -> tensor) to out_dir/<name>.npy in float32 (float64 stays
+    float64), with a _rank<r> suffix when several ranks run. A tensor whose file would exceed its equal share of
+    DUMP_BYTES is written as its elements at a fixed, seeded, sorted set of flat indices (the same for every tensor of
+    that size on every run), so the outputs of two builds can be compared element for element."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // (len(outputs) * world) - 1024          # 1 KB of each file's share kept for its header
+    for name, t in outputs.items():
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        t = t.detach()
+        n = share // (8 if dt == torch.float64 else 4)
+        if t.numel() > n:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), n, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        suffix = f"_rank{rank}" if world > 1 else ""
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), t.to(dt).cpu().numpy())
+
+
 def cpu_reference_leg(w, nnz, steps, warmup, heads):
     """The reference's CPU path (its tests' dense attention; oracle port) on a bounded sample."""
     import torch
@@ -200,13 +225,14 @@ def ring_bench(args, w, nnz, config, rank, world, local_rank):
         return (torch.rand(w["batch"] + (ch, shard), generator=g, device=dev) * 4 - 2).half()
     Q, K, V = u(w["d"]), u(w["d"]), u(w["v_d"])
     dO = u(w["v_d"])
+    out = {}                                            # what the last step returned (--dump-outputs)
 
     def ring_step():
         if not args.ring_bwd:
-            ring.ring_causal_1d(Q, K, V)
+            out["O"] = ring.ring_causal_1d(Q, K, V)
             return
-        O, l, m = ring.ring_causal_1d(Q, K, V, returning_l_m=True)
-        ring.ring_causal_1d_backward(Q, K, V, O, l, m, dO)
+        out["O"], out["l"], out["m"] = ring.ring_causal_1d(Q, K, V, returning_l_m=True)
+        out["dQ"], out["dK"], out["dV"] = ring.ring_causal_1d_backward(Q, K, V, out["O"], out["l"], out["m"], dO)
     sampler = ClockSampler(local_rank)
     sampler.launch()
     for _ in range(max(3, args.warmup)):
@@ -227,6 +253,8 @@ def ring_bench(args, w, nnz, config, rank, world, local_rank):
         dist.barrier()
     launches = int(_capi.lib.fa_launch_count(0))
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, rank, world)
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -296,6 +324,8 @@ def layout_bench(args, w, rank, world, local_rank):
         dist.barrier()
     launches = int(_capi.lib.fa_launch_count(0))
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"channel_first": y, "round_trip": x2}, rank, world)
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -321,10 +351,17 @@ def layout_bench(args, w, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"{s} is not a positive integer")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2", choices=sorted(WORKLOADS))
@@ -341,7 +378,12 @@ def main():
     ap.add_argument("--grad-precision", type=int, default=0, help="fa_set_grad_precision mode (0 auto, 1 split, 2 off)")
     ap.add_argument("--graph", action="store_true", help="replay the step as one CUDA graph (launch-bound workloads)")
     ap.add_argument("--ring-bwd", action="store_true", help="C5: time forward + ring backward")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB in all: larger outputs as a fixed, seeded sample of their elements)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -501,6 +543,11 @@ def main():
     if args.graph:
         launches = graph_launches * args.steps   # replayed from the captured graph, not re-issued by the library
     clocks = sampler.stop()
+    if args.dump_outputs:
+        outputs = {"O": O, "l": l, "m": m}
+        if not args.fwd_only:
+            outputs.update(dQ=dQ, dK=dK, dV=dV)
+        dump_outputs(args.dump_outputs, outputs, rank, world)
     ms_total = e0.elapsed_time(e1)
     kt = _capi.kernel_timings()
     if not timing_inline and not args.graph:
@@ -729,4 +776,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree and writes nothing into it
     main()
