@@ -200,7 +200,7 @@ int fa_forward(const fa_problem_t* p, const void* q, const void* k, const void* 
     e = fa::f64_dmma_forward(a, st);
   } else {
     if (a.layout != 0) return FA_EINVAL_LAYOUT;
-    if (!fa::generic_supports(a)) return FA_EINVAL_SHAPE;
+    if (!fa::generic_supports(a, false)) return FA_EINVAL_SHAPE;
     fa::g_last_path = 1;
     e = fa::generic_forward(a, st);
   }
@@ -234,7 +234,7 @@ int fa_backward(const fa_problem_t* p, const void* q, const void* k, const void*
     e = fa::f64_dmma_backward(a, st);
   } else {
     if (a.layout != 0) return FA_EINVAL_LAYOUT;
-    if (!fa::generic_supports(a)) return FA_EINVAL_SHAPE;
+    if (!fa::generic_supports(a, true)) return FA_EINVAL_SHAPE;
     fa::g_last_path = 1;
     e = fa::generic_backward(a, st);
   }
@@ -304,7 +304,7 @@ int fa_dispatch_path(const fa_problem_t* p, int is_backward, char* reason, size_
   const bool bwd = is_backward != 0;
   if (fa::g_path_override == 1) {
     say("fa_set_path_override(1): generic kernels forced");
-    return a.layout ? FA_EINVAL_LAYOUT : 1;
+    return a.layout ? FA_EINVAL_LAYOUT : fa::generic_supports(a, bwd) ? 1 : FA_EINVAL_SHAPE;
   }
   const int64_t nq = a.rule.q.total, nk = a.rule.k.total;
   const int64_t cap = 32 * int64_t(fa::sm100::kMaxTileWords);   // streamed tiles of a CTA's schedule
@@ -317,6 +317,15 @@ int fa_dispatch_path(const fa_problem_t* p, int is_backward, char* reason, size_
     say("channel-last operands are read directly only by the fp16 tensor-core kernels (channels multiples of 8 up to 128)");
     return FA_EINVAL_LAYOUT;
   }
+  if (p->d > 256 || p->v_d > 256) {
+    if (!fa::generic_supports(a, bwd)) {
+      say("more than 256 channels: batch x tiles x channel slices exceeds a 31-bit grid");
+      return FA_EINVAL_SHAPE;
+    }
+    say("more than 256 channels: channel-sliced generic kernels (each CTA owns at most 256 output channels and "
+        "recomputes S for them)");
+    return 1;
+  }
   if (p->d > max_ch || p->v_d > max_ch)
     say(p->dtype == FA_F16 ? "more than 128 channels: generic kernels" : "more than 64 channels: generic kernels");
   else if (!bwd && a.accumulate)
@@ -326,10 +335,6 @@ int fa_dispatch_path(const fa_problem_t* p, int is_backward, char* reason, size_
         "keys for the head_dim-128 forward): generic kernels; shard the sequence (K/V ring) to stay on the tensor cores");
   else
     say("batch x tiles exceeds a 31-bit grid: generic kernels");
-  if (!fa::generic_supports(a)) {
-    say("more than 256 channels: no kernel");
-    return FA_EINVAL_SHAPE;
-  }
   return 1;
 }
 

@@ -1,9 +1,13 @@
 // fa_generic.cu — the any-shape / any-dtype kernel family (SIMT, fp32 or fp64 accumulate).
 //
 // This is the engine's universal path: it accepts every (q, k, d, v_d) the reference
-// accepts up to 256 channels, every rule and sync mode, half/float/double, and is what
-// the tcgen05 kernels fall back to for shapes TMA cannot address. It is a flash-attention-2
-// style design (one CTA per Q tile, online softmax in registers, O written once) instead of
+// accepts, every rule and sync mode, half/float/double, and is what the tcgen05 kernels
+// fall back to for shapes TMA cannot address. Up to 256 channels a CTA keeps whole
+// [channels][tile] operand tiles in shared memory. Above 256 channels (KC > 0, "wide") the
+// same kernels stream the Q.K^T and dO.V^T reductions through shared memory in chunks of
+// KC channels and split the output channels across the grid: each CTA owns a slice of at
+// most 256 of them and recomputes S for it. Every output element has one writer.
+// It is a flash-attention-2 style design (one CTA per Q tile, online softmax in registers, O written once) instead of
 // the reference's K-outer loop with O/l/m read-modify-written in HBM under a spin lock
 // (reference: flash_attention/kernel/flash_attention.cu:858-1076, 1725-1950).
 //
@@ -30,6 +34,9 @@ struct FwdParams {
   int64_t batch;
   int32_t accumulate;
   FaRule rule;
+  // wide kernels (KC > 0): the grid runs slices slice_lo .. slice_lo + n_sl - 1 of O's channels, sw channels each;
+  // res = Q stays resident in shared memory whole instead of streamed in chunks
+  int32_t sw, n_sl, slice_lo, res;
 };
 
 template <typename T>
@@ -41,20 +48,27 @@ struct BwdParams {
   int32_t d, v_d, nq, nk, n_rtiles;
   int64_t batch;
   FaRule rule;
+  // wide kernels (KC > 0). dQ: n_sl slices of d, sw channels each. dK/dV: slices 0 .. n_sl_k - 1 cover dK (sw channels
+  // each), the remaining n_sl - n_sl_k cover dV (sw_v channels each). res = the resident-side operands (Q and dO, or K
+  // and V) stay in shared memory whole instead of streamed in chunks
+  int32_t sw, sw_v, n_sl, n_sl_k, res;
 };
 
 // ---- tile primitives ---------------------------------------------------------------------
 // Thread (ty, tx) of the 16x16 grid owns resident rows ty*RM..ty*RM+RM-1 (contiguous) and
 // streamed columns tx + 16*j (interleaved -> conflict-free reads of the +1 padded tile).
 
-template <typename A, int BM, int BN>
+// ADD = true adds to acc instead of overwriting it (one channel chunk of a longer reduction).
+template <typename A, int BM, int BN, bool ADD = false>
 __device__ __forceinline__ void gemm_s(const A* __restrict__ R, const A* __restrict__ S, int C,
                                        A (&acc)[BM / 16][BN / 16], int ty, int tx) {
   constexpr int RM = BM / 16, CN = BN / 16;
+  if constexpr (!ADD) {
 #pragma unroll
-  for (int i = 0; i < RM; ++i)
+    for (int i = 0; i < RM; ++i)
 #pragma unroll
-    for (int j = 0; j < CN; ++j) acc[i][j] = A(0);
+      for (int j = 0; j < CN; ++j) acc[i][j] = A(0);
+  }
   for (int c = 0; c < C; ++c) {
     A a[RM], b[CN];
 #pragma unroll
@@ -107,6 +121,29 @@ __device__ __forceinline__ void load_tile(A* __restrict__ dst, const T* __restri
   }
 }
 
+// acc = R . S^T over C channels in chunks of KC (wide kernels). R is the resident side ([C][BM] already in Rs when
+// r_res, else streamed through Rs as [KC][BM] chunks from r_src, row pitch r_n, columns r0..); S is streamed through
+// Ss as [KC][BN+1] chunks. Synchronises before each chunk, so the caller need not free Rs / Ss first. Every CTA that
+// computes the same tile runs the same products in the same order, so the result is bit-identical across slices.
+template <typename T, typename A, int BM, int BN, int KC>
+__device__ __forceinline__ void gemm_s_chunked(A* __restrict__ Rs, bool r_res, const T* __restrict__ r_src,
+                                               int64_t r_n, int64_t r0, A* __restrict__ Ss,
+                                               const T* __restrict__ s_src, int64_t s_n, int64_t s0, int C,
+                                               A (&acc)[BM / 16][BN / 16], int ty, int tx) {
+#pragma unroll
+  for (int i = 0; i < BM / 16; ++i)
+#pragma unroll
+    for (int j = 0; j < BN / 16; ++j) acc[i][j] = A(0);
+  for (int c0 = 0; c0 < C; c0 += KC) {
+    const int cc = min(KC, C - c0);
+    __syncthreads();
+    if (!r_res) load_tile<T, A>(Rs, r_src + int64_t(c0) * r_n, cc, BM, BM, r_n, r0);
+    load_tile<T, A>(Ss, s_src + int64_t(c0) * s_n, cc, BN, BN + 1, s_n, s0);
+    __syncthreads();
+    gemm_s<A, BM, BN, true>(r_res ? Rs + c0 * BM : Rs, Ss, cc, acc, ty, tx);
+  }
+}
+
 template <typename A>
 __device__ __forceinline__ A half_warp_max(A v) {
 #pragma unroll
@@ -121,26 +158,35 @@ __device__ __forceinline__ A half_warp_sum(A v) {
 }
 
 // ---- forward -----------------------------------------------------------------------------
-template <typename T, int BM, int BN, int NS>
+// KC == 0: one CTA per Q tile, all v_d output channels. KC > 0 (wide): one CTA per (Q tile, slice of O's channels).
+template <typename T, int BM, int BN, int NS, int KC = 0>
 __global__ void __launch_bounds__(NT) fwd_kernel(const FwdParams<T> p) {
   using A = typename AccOf<T>::type;
   using L = typename LOf<T>::type;
   constexpr int RM = BM / 16, CN = BN / 16;
+  constexpr bool WIDE = KC > 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  A* Qs = reinterpret_cast<A*>(smem_raw);      // [d][BM]
-  A* Ks = Qs + p.d * BM;                       // [d][BN+1]
-  A* Vs = Ks + p.d * (BN + 1);                 // [v_d][BN+1]  (also the O staging buffer)
-  A* Ps = Vs + p.v_d * (BN + 1);               // [BM][BN+1]
+  A* Qs = reinterpret_cast<A*>(smem_raw);                     // [d][BM]     (wide, streamed: [KC][BM])
+  A* Ks = Qs + (WIDE && !p.res ? KC : p.d) * BM;              // [d][BN+1]   (wide: [KC][BN+1] chunks)
+  A* Vs = Ks + (WIDE ? KC : p.d) * (BN + 1);                  // [v_d][BN+1] (wide: [sw][BN+1])  also the O staging buffer
+  A* Ps = Vs + (WIDE ? p.sw : p.v_d) * (BN + 1);              // [BM][BN+1]
 
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const int rt = p.n_rtiles - 1 - int(blockIdx.x % p.n_rtiles);  // heavy (late) tiles first
-  const int64_t b = blockIdx.x / p.n_rtiles;
+  int64_t b = blockIdx.x / p.n_rtiles;
+  int slice = 0, c_lo = 0, c_n = 0;  // wide: this CTA's output channels are c_lo .. c_lo + c_n - 1
+  if constexpr (WIDE) {
+    slice = p.slice_lo + int(b % p.n_sl);
+    b /= p.n_sl;
+    c_lo = slice * p.sw;
+    c_n = min(p.sw, p.v_d - c_lo);
+  }
   const int q0 = rt * BM;
   const int q_hi = min(q0 + BM, p.nq) - 1;
   const FaRule& rule = p.rule;
   const A scale = A(1) / sqrt(A(p.d));
 
-  load_tile<T, A>(Qs, p.q + b * p.d * int64_t(p.nq), p.d, BM, BM, p.nq, q0);
+  if (!WIDE || p.res) load_tile<T, A>(Qs, p.q + b * p.d * int64_t(p.nq), p.d, BM, BM, p.nq, q0);
 
   FaPos qpos[RM];
   A m_i[RM], l_i[RM], acc[RM][NS];
@@ -165,7 +211,8 @@ __global__ void __launch_bounds__(NT) fwd_kernel(const FwdParams<T> p) {
 #pragma unroll
           for (int s = 0; s < NS; ++s) {
             int ch = tx + 16 * s;
-            if (ch < p.v_d) acc[i][s] = to_acc<A>(p.o[(b * p.v_d + ch) * int64_t(p.nq) + qi]) * l_i[i];
+            if (ch < (WIDE ? c_n : p.v_d))
+              acc[i][s] = to_acc<A>(p.o[(b * p.v_d + (WIDE ? c_lo + ch : ch)) * int64_t(p.nq) + qi]) * l_i[i];
           }
         }
       }
@@ -180,12 +227,17 @@ __global__ void __launch_bounds__(NT) fwd_kernel(const FwdParams<T> p) {
     const int cls = fa_classify(rule, q0, q_hi, k0, k_hi);
     if (cls == FA_TILE_SKIP) continue;
     __syncthreads();
-    load_tile<T, A>(Ks, p.k + b * p.d * int64_t(p.nk), p.d, BN, BN + 1, p.nk, k0);
-    load_tile<T, A>(Vs, p.v + b * p.v_d * int64_t(p.nk), p.v_d, BN, BN + 1, p.nk, k0);
-    __syncthreads();
-
     A s[RM][CN];
-    gemm_s<A, BM, BN>(Qs, Ks, p.d, s, ty, tx);
+    if constexpr (!WIDE) {
+      load_tile<T, A>(Ks, p.k + b * p.d * int64_t(p.nk), p.d, BN, BN + 1, p.nk, k0);
+      load_tile<T, A>(Vs, p.v + b * p.v_d * int64_t(p.nk), p.v_d, BN, BN + 1, p.nk, k0);
+      __syncthreads();
+      gemm_s<A, BM, BN>(Qs, Ks, p.d, s, ty, tx);
+    } else {
+      load_tile<T, A>(Vs, p.v + (b * p.v_d + c_lo) * int64_t(p.nk), c_n, BN, BN + 1, p.nk, k0);
+      gemm_s_chunked<T, A, BM, BN, KC>(Qs, p.res, p.q + b * p.d * int64_t(p.nq), p.nq, q0, Ks,
+                                       p.k + b * p.d * int64_t(p.nk), p.nk, k0, p.d, s, ty, tx);
+    }
 
 #pragma unroll
     for (int j = 0; j < CN; ++j) {
@@ -226,22 +278,23 @@ __global__ void __launch_bounds__(NT) fwd_kernel(const FwdParams<T> p) {
       for (int j = 0; j < CN; ++j) Ps[(ty * RM + i) * (BN + 1) + tx + 16 * j] = s[i][j];
     }
     __syncthreads();
-    gemm_pv<A, BM, BN, NS>(Ps, Vs, p.v_d, acc, ty, tx);
+    gemm_pv<A, BM, BN, NS>(Ps, Vs, WIDE ? c_n : p.v_d, acc, ty, tx);
   }
 
   // epilogue: O = acc / l staged through smem so that the store is coalesced along q
   __syncthreads();
-  A* Os = Vs;  // [v_d][BM+1]  (BM == BN)
+  A* Os = Vs;  // [c_n][BM+1]  (BM == BN)
 #pragma unroll
   for (int i = 0; i < RM; ++i) {
     const A inv = l_i[i] > A(0) ? A(1) / l_i[i] : A(0);
 #pragma unroll
     for (int s = 0; s < NS; ++s) {
       int ch = tx + 16 * s;
-      if (ch < p.v_d) Os[ch * (BM + 1) + ty * RM + i] = acc[i][s] * inv;
+      if (ch < (WIDE ? c_n : p.v_d)) Os[ch * (BM + 1) + ty * RM + i] = acc[i][s] * inv;
     }
     const int qi = q0 + ty * RM + i;
-    if (tx == 0 && qi < p.nq) {
+    // every slice computes the same m and l bit for bit; slice 0 stores them
+    if (tx == 0 && qi < p.nq && (!WIDE || slice == 0)) {
       if (l_i[i] > A(0)) {
         // m is stored in T; l is re-expressed against the rounded m so that
         // exp(s - m_T) / l_out reproduces the exact probabilities in the backward.
@@ -256,8 +309,8 @@ __global__ void __launch_bounds__(NT) fwd_kernel(const FwdParams<T> p) {
     }
   }
   __syncthreads();
-  T* og = p.o + b * p.v_d * int64_t(p.nq);
-  const int total = p.v_d * BM;
+  T* og = p.o + (WIDE ? b * p.v_d + c_lo : b * p.v_d) * int64_t(p.nq);
+  const int total = (WIDE ? c_n : p.v_d) * BM;
   for (int idx = threadIdx.x; idx < total; idx += NT) {
     int ch = idx / BM, r = idx - ch * BM;
     if (q0 + r < p.nq) og[int64_t(ch) * p.nq + q0 + r] = from_acc<T>(Os[ch * (BM + 1) + r]);
@@ -288,27 +341,38 @@ __global__ void bwd_prep_kernel(const T* __restrict__ o, const T* __restrict__ d
 }
 
 // ---- backward dQ: one CTA per Q tile, streams K/V tiles ------------------------------------
-template <typename T, int BM, int BN, int NS>
+// KC > 0 (wide): one CTA per (Q tile, slice of dQ's channels).
+template <typename T, int BM, int BN, int NS, int KC = 0>
 __global__ void __launch_bounds__(NT) bwd_dq_kernel(const BwdParams<T> p) {
   using A = typename AccOf<T>::type;
   constexpr int RM = BM / 16, CN = BN / 16;
+  constexpr bool WIDE = KC > 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  A* Qs = reinterpret_cast<A*>(smem_raw);  // [d][BM]
-  A* dOs = Qs + p.d * BM;                  // [v_d][BM]
-  A* Ks = dOs + p.v_d * BM;                // [d][BN+1]   (also dQ staging)
-  A* Vs = Ks + p.d * (BN + 1);             // [v_d][BN+1]
-  A* Ds = Vs + p.v_d * (BN + 1);           // [BM][BN+1]  dS tile
+  A* Qs = reinterpret_cast<A*>(smem_raw);           // [d][BM]     (wide, streamed: [KC][BM])
+  A* dOs = Qs + (WIDE && !p.res ? KC : p.d) * BM;   // [v_d][BM]   (wide, streamed: [KC][BM])
+  A* Ks = dOs + (WIDE && !p.res ? KC : p.v_d) * BM; // [d][BN+1]   (wide: the K slice [sw][BN+1])  also dQ staging
+  A* Vs = Ks + (WIDE ? p.sw : p.d) * (BN + 1);      // [v_d][BN+1] (wide: K and V chunks [KC][BN+1])
+  A* Ds = Vs + (WIDE ? KC : p.v_d) * (BN + 1);      // [BM][BN+1]  dS tile
 
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const int rt = p.n_rtiles - 1 - int(blockIdx.x % p.n_rtiles);
-  const int64_t b = blockIdx.x / p.n_rtiles;
+  int64_t b = blockIdx.x / p.n_rtiles;
+  int c_lo = 0, c_n = 0;  // wide: this CTA's dQ channels are c_lo .. c_lo + c_n - 1
+  if constexpr (WIDE) {
+    const int slice = int(b % p.n_sl);
+    b /= p.n_sl;
+    c_lo = slice * p.sw;
+    c_n = min(p.sw, p.d - c_lo);
+  }
   const int q0 = rt * BM;
   const int q_hi = min(q0 + BM, p.nq) - 1;
   const FaRule& rule = p.rule;
   const A scale = A(1) / sqrt(A(p.d));
 
-  load_tile<T, A>(Qs, p.q + b * p.d * int64_t(p.nq), p.d, BM, BM, p.nq, q0);
-  load_tile<T, A>(dOs, p.d_o + b * p.v_d * int64_t(p.nq), p.v_d, BM, BM, p.nq, q0);
+  if (!WIDE || p.res) {
+    load_tile<T, A>(Qs, p.q + b * p.d * int64_t(p.nq), p.d, BM, BM, p.nq, q0);
+    load_tile<T, A>(dOs, p.d_o + b * p.v_d * int64_t(p.nq), p.v_d, BM, BM, p.nq, q0);
+  }
 
   FaPos qpos[RM];
   A lse[RM], dsum[RM], dq[RM][NS];
@@ -330,12 +394,20 @@ __global__ void __launch_bounds__(NT) bwd_dq_kernel(const BwdParams<T> p) {
     const int cls = fa_classify(rule, q0, q_hi, k0, k_hi);
     if (cls == FA_TILE_SKIP) continue;
     __syncthreads();
-    load_tile<T, A>(Ks, p.k + b * p.d * int64_t(p.nk), p.d, BN, BN + 1, p.nk, k0);
-    load_tile<T, A>(Vs, p.v + b * p.v_d * int64_t(p.nk), p.v_d, BN, BN + 1, p.nk, k0);
-    __syncthreads();
     A s[RM][CN], dp[RM][CN];
-    gemm_s<A, BM, BN>(Qs, Ks, p.d, s, ty, tx);
-    gemm_s<A, BM, BN>(dOs, Vs, p.v_d, dp, ty, tx);
+    if constexpr (!WIDE) {
+      load_tile<T, A>(Ks, p.k + b * p.d * int64_t(p.nk), p.d, BN, BN + 1, p.nk, k0);
+      load_tile<T, A>(Vs, p.v + b * p.v_d * int64_t(p.nk), p.v_d, BN, BN + 1, p.nk, k0);
+      __syncthreads();
+      gemm_s<A, BM, BN>(Qs, Ks, p.d, s, ty, tx);
+      gemm_s<A, BM, BN>(dOs, Vs, p.v_d, dp, ty, tx);
+    } else {
+      load_tile<T, A>(Ks, p.k + (b * p.d + c_lo) * int64_t(p.nk), c_n, BN, BN + 1, p.nk, k0);
+      gemm_s_chunked<T, A, BM, BN, KC>(Qs, p.res, p.q + b * p.d * int64_t(p.nq), p.nq, q0, Vs,
+                                       p.k + b * p.d * int64_t(p.nk), p.nk, k0, p.d, s, ty, tx);
+      gemm_s_chunked<T, A, BM, BN, KC>(dOs, p.res, p.d_o + b * p.v_d * int64_t(p.nq), p.nq, q0, Vs,
+                                       p.v + b * p.v_d * int64_t(p.nk), p.nk, k0, p.v_d, dp, ty, tx);
+    }
 #pragma unroll
     for (int j = 0; j < CN; ++j) {
       const int kj = k0 + tx + 16 * j;
@@ -349,20 +421,20 @@ __global__ void __launch_bounds__(NT) bwd_dq_kernel(const BwdParams<T> p) {
       }
     }
     __syncthreads();
-    gemm_pv<A, BM, BN, NS>(Ds, Ks, p.d, dq, ty, tx);
+    gemm_pv<A, BM, BN, NS>(Ds, Ks, WIDE ? c_n : p.d, dq, ty, tx);
   }
   __syncthreads();
-  A* Os = Ks;  // [d][BM+1]
+  A* Os = Ks;  // [d][BM+1]  (wide: [c_n][BM+1])
 #pragma unroll
   for (int i = 0; i < RM; ++i)
 #pragma unroll
     for (int s = 0; s < NS; ++s) {
       int ch = tx + 16 * s;
-      if (ch < p.d) Os[ch * (BM + 1) + ty * RM + i] = dq[i][s];
+      if (ch < (WIDE ? c_n : p.d)) Os[ch * (BM + 1) + ty * RM + i] = dq[i][s];
     }
   __syncthreads();
-  T* og = p.d_q + b * p.d * int64_t(p.nq);
-  const int total = p.d * BM;
+  T* og = p.d_q + (WIDE ? b * p.d + c_lo : b * p.d) * int64_t(p.nq);
+  const int total = (WIDE ? c_n : p.d) * BM;
   for (int idx = threadIdx.x; idx < total; idx += NT) {
     int ch = idx / BM, r = idx - ch * BM;
     if (q0 + r < p.nq) og[int64_t(ch) * p.nq + q0 + r] = from_acc<T>(Os[ch * (BM + 1) + r]);
@@ -370,34 +442,49 @@ __global__ void __launch_bounds__(NT) bwd_dq_kernel(const BwdParams<T> p) {
 }
 
 // ---- backward dK/dV: one CTA per K tile (resident), streams Q/dO tiles ---------------------
-template <typename T, int BM, int BN, int NS>
+// KC > 0 (wide): one CTA per (K tile, slice of the concatenated dK | dV channels). A slice lies in dK or in dV, never
+// across both: a dV slice needs P only, a dK slice dS (and so dP = V . dO^T as well).
+template <typename T, int BM, int BN, int NS, int KC = 0>
 __global__ void __launch_bounds__(NT) bwd_dkdv_kernel(const BwdParams<T> p) {
   using A = typename AccOf<T>::type;
   constexpr int RM = BM / 16, CN = BN / 16;
+  constexpr bool WIDE = KC > 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  A* Ks = reinterpret_cast<A*>(smem_raw);  // [d][BM]     resident keys
-  A* Vs = Ks + p.d * BM;                   // [v_d][BM]
-  A* Qs = Vs + p.v_d * BM;                 // [d][BN+1]   streamed queries (also dK staging)
-  A* dOs = Qs + p.d * (BN + 1);            // [v_d][BN+1] (also dV staging)
-  A* Ps = dOs + p.v_d * (BN + 1);          // [BM][BN+1]  P^T
-  A* Ds = Ps + BM * (BN + 1);              // [BM][BN+1]  dS^T
-  A* lse_s = Ds + BM * (BN + 1);           // [BN]
-  A* dsum_s = lse_s + BN;                  // [BN]
+  A* Ks = reinterpret_cast<A*>(smem_raw);                     // [d][BM]     resident keys  (wide, streamed: [KC][BM])
+  A* Vs = Ks + (WIDE && !p.res ? KC : p.d) * BM;              // [v_d][BM]   (wide, streamed: [KC][BM])
+  A* Qs = Vs + (WIDE && !p.res ? KC : p.v_d) * BM;            // [d][BN+1]   streamed queries (also dK staging)
+                                                              //   (wide: the Q or dO slice [max(sw, sw_v)][BN+1])
+  A* dOs = Qs + (WIDE ? max(p.sw, p.sw_v) : p.d) * (BN + 1);  // [v_d][BN+1] (also dV staging)
+                                                              //   (wide: Q and dO chunks [KC][BN+1])
+  A* Ps = dOs + (WIDE ? KC : p.v_d) * (BN + 1);               // [BM][BN+1]  P^T
+  A* Ds = Ps + BM * (BN + 1);                                 // [BM][BN+1]  dS^T
+  A* lse_s = Ds + BM * (BN + 1);                              // [BN]
+  A* dsum_s = lse_s + BN;                                     // [BN]
 
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const int rt = int(blockIdx.x % p.n_rtiles);  // early key tiles are the heavy ones under causal
-  const int64_t b = blockIdx.x / p.n_rtiles;
+  int64_t b = blockIdx.x / p.n_rtiles;
+  int slice = 0;
+  if constexpr (WIDE) {
+    slice = int(b % p.n_sl);
+    b /= p.n_sl;
+  }
+  const bool is_dk = !WIDE || slice < p.n_sl_k;      // wide: this CTA writes dK channels (else dV channels)
+  const int c_lo = !WIDE ? 0 : is_dk ? slice * p.sw : (slice - p.n_sl_k) * p.sw_v;
+  const int c_n = !WIDE ? 0 : is_dk ? min(p.sw, p.d - c_lo) : min(p.sw_v, p.v_d - c_lo);
   const int k0 = rt * BM;
   const int k_hi = min(k0 + BM, p.nk) - 1;
   const FaRule& rule = p.rule;
   const A scale = A(1) / sqrt(A(p.d));
 
-  load_tile<T, A>(Ks, p.k + b * p.d * int64_t(p.nk), p.d, BM, BM, p.nk, k0);
-  load_tile<T, A>(Vs, p.v + b * p.v_d * int64_t(p.nk), p.v_d, BM, BM, p.nk, k0);
+  if (!WIDE || p.res) {
+    load_tile<T, A>(Ks, p.k + b * p.d * int64_t(p.nk), p.d, BM, BM, p.nk, k0);
+    load_tile<T, A>(Vs, p.v + b * p.v_d * int64_t(p.nk), p.v_d, BM, BM, p.nk, k0);
+  }
 
   FaPos kpos[RM];
   bool kvalid[RM];
-  A dk[RM][NS], dv[RM][NS];
+  A dk[RM][NS], dv[RM][NS];  // wide: dk is the slice's accumulator, dv is unused
 #pragma unroll
   for (int i = 0; i < RM; ++i) {
     int ki = k0 + ty * RM + i;
@@ -415,18 +502,37 @@ __global__ void __launch_bounds__(NT) bwd_dkdv_kernel(const BwdParams<T> p) {
     const int cls = fa_classify(rule, q0, q_hi, k0, k_hi);
     if (cls == FA_TILE_SKIP) continue;
     __syncthreads();
-    load_tile<T, A>(Qs, p.q + b * p.d * int64_t(p.nq), p.d, BN, BN + 1, p.nq, q0);
-    load_tile<T, A>(dOs, p.d_o + b * p.v_d * int64_t(p.nq), p.v_d, BN, BN + 1, p.nq, q0);
+    if constexpr (!WIDE) {
+      load_tile<T, A>(Qs, p.q + b * p.d * int64_t(p.nq), p.d, BN, BN + 1, p.nq, q0);
+      load_tile<T, A>(dOs, p.d_o + b * p.v_d * int64_t(p.nq), p.v_d, BN, BN + 1, p.nq, q0);
+    } else {
+      const T* src = is_dk ? p.q + (b * p.d + c_lo) * int64_t(p.nq) : p.d_o + (b * p.v_d + c_lo) * int64_t(p.nq);
+      load_tile<T, A>(Qs, src, c_n, BN, BN + 1, p.nq, q0);
+    }
     if (threadIdx.x < BN) {
       int qi = q0 + threadIdx.x;
       bool v = qi < p.nq;
       lse_s[threadIdx.x] = v ? p.lse[b * p.nq + qi] : -neg_inf<A>();
       dsum_s[threadIdx.x] = v ? p.dsum[b * p.nq + qi] : A(0);
     }
-    __syncthreads();
     A st[RM][CN], dpt[RM][CN];
-    gemm_s<A, BM, BN>(Ks, Qs, p.d, st, ty, tx);
-    gemm_s<A, BM, BN>(Vs, dOs, p.v_d, dpt, ty, tx);
+    if constexpr (!WIDE) {
+      __syncthreads();
+      gemm_s<A, BM, BN>(Ks, Qs, p.d, st, ty, tx);
+      gemm_s<A, BM, BN>(Vs, dOs, p.v_d, dpt, ty, tx);
+    } else {
+      gemm_s_chunked<T, A, BM, BN, KC>(Ks, p.res, p.k + b * p.d * int64_t(p.nk), p.nk, k0, dOs,
+                                       p.q + b * p.d * int64_t(p.nq), p.nq, q0, p.d, st, ty, tx);
+      if (is_dk) {
+        gemm_s_chunked<T, A, BM, BN, KC>(Vs, p.res, p.v + b * p.v_d * int64_t(p.nk), p.nk, k0, dOs,
+                                         p.d_o + b * p.v_d * int64_t(p.nq), p.nq, q0, p.v_d, dpt, ty, tx);
+      } else {
+#pragma unroll
+        for (int i = 0; i < RM; ++i)
+#pragma unroll
+          for (int j = 0; j < CN; ++j) dpt[i][j] = A(0);
+      }
+    }
 #pragma unroll
     for (int j = 0; j < CN; ++j) {
       const int col = tx + 16 * j;
@@ -443,10 +549,31 @@ __global__ void __launch_bounds__(NT) bwd_dkdv_kernel(const BwdParams<T> p) {
       }
     }
     __syncthreads();
-    gemm_pv<A, BM, BN, NS>(Ps, dOs, p.v_d, dv, ty, tx);
-    gemm_pv<A, BM, BN, NS>(Ds, Qs, p.d, dk, ty, tx);
+    if constexpr (!WIDE) {
+      gemm_pv<A, BM, BN, NS>(Ps, dOs, p.v_d, dv, ty, tx);
+      gemm_pv<A, BM, BN, NS>(Ds, Qs, p.d, dk, ty, tx);
+    } else {
+      gemm_pv<A, BM, BN, NS>(is_dk ? Ds : Ps, Qs, c_n, dk, ty, tx);
+    }
   }
   __syncthreads();
+  if constexpr (WIDE) {
+    A* Os = Qs;  // [c_n][BM+1]
+#pragma unroll
+    for (int i = 0; i < RM; ++i)
+#pragma unroll
+      for (int s = 0; s < NS; ++s) {
+        int ch = tx + 16 * s;
+        if (ch < c_n) Os[ch * (BM + 1) + ty * RM + i] = dk[i][s];
+      }
+    __syncthreads();
+    T* og = is_dk ? p.d_k + (b * p.d + c_lo) * int64_t(p.nk) : p.d_v + (b * p.v_d + c_lo) * int64_t(p.nk);
+    for (int idx = threadIdx.x; idx < c_n * BM; idx += NT) {
+      int ch = idx / BM, r = idx - ch * BM;
+      if (k0 + r < p.nk) og[int64_t(ch) * p.nk + k0 + r] = from_acc<T>(Os[ch * (BM + 1) + r]);
+    }
+    return;
+  }
   A* Ok = Qs;   // [d][BM+1]
   A* Ov = dOs;  // [v_d][BM+1]
 #pragma unroll
@@ -506,6 +633,138 @@ struct Tiles {
   static constexpr int kSmall = kBig / 2;
 };
 
+// ---- wide heads: more than 256 channels ------------------------------------------------------
+// Each CTA owns a slice of at most 16 x NS <= 256 output channels, so the register accumulators keep the shape of the
+// SMALL tiles; the grid is batch x row tiles x slices. Every slice recomputes S (and dP), so the host picks, among the
+// instantiated NS, the slicing with the least arithmetic.
+constexpr int kWideKC = 64;                 // channels per chunk of the streamed Q.K^T / dO.V^T reductions
+constexpr int kWideNS[] = {4, 10, 16};   // instantiated accumulator widths (16 x NS channels per slice)
+
+struct Slices {
+  int n, w;  // n slices of w channels (a multiple of 16; the last slice may be narrower)
+};
+static Slices slices(int C, int ns) {
+  const int u = (C + 15) / 16, n = (u + ns - 1) / ns;
+  return {n, 16 * ((u + n - 1) / n)};
+}
+
+enum WideKind { kWideFwd, kWideDq, kWideDkdv };
+struct WidePlan {
+  int ns;
+  Slices s, v;  // forward: O's channels; dQ: d; dK/dV: s = dK's channels, v = dV's channels
+  bool res;     // the resident-side operands stay whole in shared memory
+  size_t smem;
+  int n_sl() const { return s.n + v.n; }
+};
+
+static WidePlan wide_plan(WideKind kind, int d, int v_d, int BM, size_t acc_bytes) {
+  WidePlan best{};
+  int64_t best_cost = -1;
+  for (int ns : kWideNS) {
+    WidePlan w{};
+    w.ns = ns;
+    int64_t cost;
+    if (kind == kWideFwd) {
+      w.s = slices(v_d, ns);
+      cost = int64_t(w.s.n) * (d + 16 * ns);
+    } else if (kind == kWideDq) {
+      w.s = slices(d, ns);
+      cost = int64_t(w.s.n) * (int64_t(d) + v_d + 16 * ns);
+    } else {
+      w.s = slices(d, ns);
+      w.v = slices(v_d, ns);
+      cost = int64_t(w.s.n) * (int64_t(d) + v_d + 16 * ns) + int64_t(w.v.n) * (d + 16 * ns);
+    }
+    if (best_cost < 0 || cost <= best_cost) {
+      best = w;
+      best_cost = cost;
+    }
+  }
+  const size_t P = BM + 1, KC = kWideKC;
+  const size_t res_rows = kind == kWideFwd ? size_t(d) : size_t(d) + v_d;
+  const size_t chunk_rows = kind == kWideFwd ? KC : 2 * KC;
+  const size_t other = kind == kWideFwd ? (KC + best.s.w + BM) * P
+                       : kind == kWideDq ? (best.s.w + KC + BM) * P
+                                         : (std::max(best.s.w, best.v.w) + KC + 2 * BM) * P + 2 * BM;
+  const size_t resident = acc_bytes * (res_rows * BM + other);
+  best.res = resident <= kSmemMax / 2;  // resident only where two CTAs still fit an SM
+  best.smem = best.res ? resident : acc_bytes * (chunk_rows * BM + other);
+  return best;
+}
+
+template <typename T>
+static WidePlan wide_plan_t(WideKind kind, int d, int v_d) {
+  return wide_plan(kind, d, v_d, Tiles<T>::kSmall, sizeof(typename AccOf<T>::type));
+}
+
+// batch x row tiles x slices of every launch of the call fits a 31-bit grid
+template <typename T>
+static bool wide_grid_fits(const LaunchArgs& a, bool backward) {
+  constexpr int BM = Tiles<T>::kSmall;
+  const int64_t rq = (int64_t(a.rule.q.total) + BM - 1) / BM, rk = (int64_t(a.rule.k.total) + BM - 1) / BM;
+  auto fits = [&](int64_t tiles, const WidePlan& w) { return a.batch <= 0x7fffffffLL / std::max<int64_t>(1, tiles * w.n_sl()); };
+  if (!backward) return fits(rq, wide_plan_t<T>(kWideFwd, a.d, a.v_d));
+  return fits(rq, wide_plan_t<T>(kWideDq, a.d, a.v_d)) && fits(rk, wide_plan_t<T>(kWideDkdv, a.d, a.v_d));
+}
+
+template <typename T>
+static cudaError_t forward_wide(FwdParams<T> p, cudaStream_t stream) {
+  constexpr int BM = Tiles<T>::kSmall, KC = kWideKC;
+  const WidePlan w = wide_plan_t<T>(kWideFwd, p.d, p.v_d);
+  p.n_rtiles = (p.nq + BM - 1) / BM;
+  p.sw = w.s.w;
+  p.res = w.res;
+  auto run = [&](int lo, int n) -> cudaError_t {
+    p.slice_lo = lo;
+    p.n_sl = n;
+    const int64_t grid = p.batch * p.n_rtiles * n;
+    switch (w.ns) {
+      case 4: return launch("generic_fwd_wide", fwd_kernel<T, BM, BM, 4, KC>, p, grid, w.smem, stream);
+      case 10: return launch("generic_fwd_wide", fwd_kernel<T, BM, BM, 10, KC>, p, grid, w.smem, stream);
+      default: return launch("generic_fwd_wide", fwd_kernel<T, BM, BM, 16, KC>, p, grid, w.smem, stream);
+    }
+  };
+  // accumulate = 1: every slice reads the incoming m and l, and slice 0 overwrites them, so slice 0 runs in a launch
+  // of its own after the others
+  if (p.accumulate && w.s.n > 1) {
+    cudaError_t e = run(1, w.s.n - 1);
+    if (e != cudaSuccess) return e;
+    return run(0, 1);
+  }
+  return run(0, w.s.n);
+}
+
+template <typename T>
+static cudaError_t backward_wide(BwdParams<T> p, cudaStream_t stream) {
+  constexpr int BM = Tiles<T>::kSmall, KC = kWideKC;
+  const WidePlan wq = wide_plan_t<T>(kWideDq, p.d, p.v_d);
+  p.n_rtiles = (p.nq + BM - 1) / BM;
+  p.sw = wq.s.w;
+  p.n_sl = wq.n_sl();
+  p.res = wq.res;
+  int64_t grid = p.batch * p.n_rtiles * p.n_sl;
+  cudaError_t e;
+  switch (wq.ns) {
+    case 4: e = launch("generic_bwd_dq_wide", bwd_dq_kernel<T, BM, BM, 4, KC>, p, grid, wq.smem, stream); break;
+    case 10: e = launch("generic_bwd_dq_wide", bwd_dq_kernel<T, BM, BM, 10, KC>, p, grid, wq.smem, stream); break;
+    default: e = launch("generic_bwd_dq_wide", bwd_dq_kernel<T, BM, BM, 16, KC>, p, grid, wq.smem, stream); break;
+  }
+  if (e != cudaSuccess) return e;
+  const WidePlan wk = wide_plan_t<T>(kWideDkdv, p.d, p.v_d);
+  p.n_rtiles = (p.nk + BM - 1) / BM;
+  p.sw = wk.s.w;
+  p.sw_v = wk.v.w;
+  p.n_sl = wk.n_sl();
+  p.n_sl_k = wk.s.n;
+  p.res = wk.res;
+  grid = p.batch * p.n_rtiles * p.n_sl;
+  switch (wk.ns) {
+    case 4: return launch("generic_bwd_dkdv_wide", bwd_dkdv_kernel<T, BM, BM, 4, KC>, p, grid, wk.smem, stream);
+    case 10: return launch("generic_bwd_dkdv_wide", bwd_dkdv_kernel<T, BM, BM, 10, KC>, p, grid, wk.smem, stream);
+    default: return launch("generic_bwd_dkdv_wide", bwd_dkdv_kernel<T, BM, BM, 16, KC>, p, grid, wk.smem, stream);
+  }
+}
+
 template <typename T>
 cudaError_t forward_t(const LaunchArgs& a, cudaStream_t stream) {
   FwdParams<T> p;
@@ -513,6 +772,7 @@ cudaError_t forward_t(const LaunchArgs& a, cudaStream_t stream) {
   p.o = (T*)a.o; p.l = (typename LOf<T>::type*)a.l; p.m = (T*)a.m;
   p.d = a.d; p.v_d = a.v_d; p.nq = a.rule.q.total; p.nk = a.rule.k.total;
   p.batch = a.batch; p.accumulate = a.accumulate; p.rule = a.rule;
+  if (std::max(a.d, a.v_d) > 256) return forward_wide<T>(p, stream);
   constexpr int BIG = Tiles<T>::kBig, SMALL = Tiles<T>::kSmall;
   const int ns = (a.v_d + 15) / 16;
 #define FA_FWD(BM_, NS_)                                                                   \
@@ -556,6 +816,7 @@ cudaError_t backward_t(const LaunchArgs& a, cudaStream_t stream) {
     }
     if (e != cudaSuccess) return e;
   }
+  if (std::max(a.d, a.v_d) > 256) return backward_wide<T>(p, stream);
   constexpr int BIG = Tiles<T>::kBig, SMALL = Tiles<T>::kSmall;
   const int ns = (std::max(a.d, a.v_d) + 15) / 16;
 #define FA_BWD(BM_, NS_)                                                                      \
@@ -578,7 +839,15 @@ cudaError_t backward_t(const LaunchArgs& a, cudaStream_t stream) {
 
 }  // namespace generic
 
-bool generic_supports(const LaunchArgs& a) { return a.layout == 0 && a.d <= 256 && a.v_d <= 256; }
+bool generic_supports(const LaunchArgs& a, bool backward) {
+  if (a.layout != 0) return false;
+  if (a.d <= 256 && a.v_d <= 256) return true;
+  switch (a.dtype) {
+    case 0: return generic::wide_grid_fits<__half>(a, backward);
+    case 1: return generic::wide_grid_fits<float>(a, backward);
+    default: return generic::wide_grid_fits<double>(a, backward);
+  }
+}
 
 size_t generic_workspace_bytes(int dtype, int64_t batch, int64_t nq, bool backward) {
   if (!backward) return 0;

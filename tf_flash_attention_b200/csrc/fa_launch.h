@@ -51,8 +51,9 @@ struct ScopedKernel {
   int slot_;
 };
 
-// generic SIMT family (fa_generic.cu)
-bool generic_supports(const LaunchArgs& a);
+// generic SIMT family (fa_generic.cu). Any channel count; above 256 channels the grid (batch x row tiles x channel
+// slices) must fit 31 bits, for the forward or for both backward kernels.
+bool generic_supports(const LaunchArgs& a, bool backward);
 size_t generic_workspace_bytes(int dtype, int64_t batch, int64_t nq, bool backward);
 cudaError_t generic_forward(const LaunchArgs& a, cudaStream_t stream);
 cudaError_t generic_backward(const LaunchArgs& a, cudaStream_t stream);
