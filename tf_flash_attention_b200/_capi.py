@@ -10,7 +10,7 @@ import os
 _HERE = os.path.abspath(os.path.dirname(__file__))
 LIB_PATH = os.environ.get("FA_B200_LIB") or os.path.join(_HERE, "libfa_b200.so")  # env override: developer A/B builds
 
-FA_F16, FA_F32, FA_F64 = 0, 1, 2
+FA_F16, FA_F32, FA_F64, FA_BF16 = 0, 1, 2, 3
 FA_RING_HANDLE_BYTES = 128
 RULES = {"full": 0, "causal": 1, "local": 2}
 SYNC_MODES = {"none_front": 0, "scale_front": 1, "scale_end": 2}

@@ -52,7 +52,7 @@ namespace {
 
 int make_rule(const fa_problem_t* p, FaRule* r) {
   if (!p) return FA_EINVAL_NULL;
-  if (p->dtype < 0 || p->dtype > 2) return FA_EINVAL_DTYPE;
+  if (p->dtype < FA_F16 || p->dtype > FA_BF16) return FA_EINVAL_DTYPE;
   if (p->seq_dims != 1 && p->seq_dims != 2) return FA_EINVAL_SEQ_DIMS;
   if (p->d < 1 || p->v_d < 1 || p->batch < 0) return FA_EINVAL_SHAPE;
   return fa_make_rule(p->seq_dims, p->rule, p->window_size, p->log2_stride_size, p->is_causal,
@@ -60,7 +60,9 @@ int make_rule(const fa_problem_t* p, FaRule* r) {
                       p->q_full_len, p->k_full_len, r);
 }
 
-size_t elt(int dtype) { return dtype == FA_F16 ? 2 : dtype == FA_F32 ? 4 : 8; }
+// fp16 and bf16 share the tcgen05 16-bit family and every size rule
+bool is16(int dtype) { return dtype == FA_F16 || dtype == FA_BF16; }
+size_t elt(int dtype) { return is16(dtype) ? 2 : dtype == FA_F32 ? 4 : 8; }
 size_t l_elt(int dtype) { return dtype == FA_F64 ? 8 : 4; }
 
 int cuda_fail(cudaError_t e) {
@@ -96,7 +98,7 @@ const char* fa_strerror(int s) {
   switch (s) {
     case FA_OK: return "ok";
     case FA_EINVAL_NULL: return "null argument";
-    case FA_EINVAL_DTYPE: return "unsupported dtype (expected float16, float32 or float64)";
+    case FA_EINVAL_DTYPE: return "unsupported dtype (expected float16, float32, float64 or bfloat16)";
     case FA_EINVAL_SEQ_DIMS: return "sequence dims must be 1 or 2";
     case FA_EINVAL_RULE: return "unknown masking rule";
     case FA_EINVAL_SYNC_MODE: return "Unsupported sync_mode";
@@ -111,7 +113,7 @@ const char* fa_strerror(int s) {
     case FA_EINVAL_BATCH: return "The batch shape of all inputs should be equal";
     case FA_EINVAL_SEQ_SHAPE: return "The sequence shapes are inconsistent";
     case FA_EINVAL_LAYOUT:
-      return "channel-last operands are read directly only by the fp16 tensor-core kernels (channels multiples of 8 up "
+      return "channel-last operands are read directly only by the 16-bit tensor-core kernels (channels multiples of 8 up "
              "to 128, 16-byte-aligned tensors, heads >= 1 dividing batch); use fa_layout_transpose otherwise";
     case FA_ECUDA: return "CUDA error (see fa_last_cuda_error)";
     case FA_ENODEVICE: return "no sm_100 CUDA device is current";
@@ -157,7 +159,7 @@ size_t fa_workspace_bytes(const fa_problem_t* p, int is_backward) {
   size_t g = fa::generic_workspace_bytes(p->dtype, p->batch, a.rule.q.total, is_backward != 0);
   size_t s = 0;
   a.variant = fa::g_path_override;
-  if (p->dtype == FA_F16) s = fa::sm100_f16_workspace_bytes(a, is_backward != 0);
+  if (is16(p->dtype)) s = fa::sm100_f16_workspace_bytes(a, is_backward != 0);
   if (p->dtype == FA_F32 && is_backward && fa::g_path_override != 1) {
     fa::LaunchArgs probe = a;
     probe.workspace = reinterpret_cast<void*>(uintptr_t(256));   // a probe: only shape / size rules are evaluated
@@ -189,7 +191,7 @@ int fa_forward(const fa_problem_t* p, const void* q, const void* k, const void* 
   a.variant = fa::g_path_override;
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e;
-  if (fa::g_path_override != 1 && p->dtype == FA_F16 && fa::sm100_f16_forward_supports(a)) {
+  if (fa::g_path_override != 1 && is16(p->dtype) && fa::sm100_f16_forward_supports(a)) {
     fa::g_last_path = 2;
     e = fa::sm100_f16_forward(a, st);
   } else if (fa::g_path_override != 1 && p->dtype == FA_F32 && fa::sm100_f32_forward_supports(a)) {
@@ -223,7 +225,7 @@ int fa_backward(const fa_problem_t* p, const void* q, const void* k, const void*
   a.variant = fa::g_path_override;
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e;
-  if (fa::g_path_override != 1 && p->dtype == FA_F16 && fa::sm100_f16_backward_supports(a)) {
+  if (fa::g_path_override != 1 && is16(p->dtype) && fa::sm100_f16_backward_supports(a)) {
     fa::g_last_path = 2;
     e = fa::sm100_f16_backward(a, st);
   } else if (fa::g_path_override != 1 && p->dtype == FA_F32 && fa::sm100_f32_backward_supports(a)) {
@@ -264,7 +266,7 @@ int fa_backward_accumulate_supported(const fa_problem_t* p, int64_t dq_fold) {
   if (!p || fill_accumulate_args(p, dummy, dummy, dummy, dummy, dummy, dummy, dummy, dummy, dummy, dummy, dq_fold, dummy,
                                  ~size_t(0), &a))
     return 0;
-  return (p->dtype == FA_F16 && fa::g_path_override != 1 && p->batch > 0 && fa::sm100_f16_backward_accumulate_supports(a)) ? 1 : 0;
+  return (is16(p->dtype) && fa::g_path_override != 1 && p->batch > 0 && fa::sm100_f16_backward_accumulate_supports(a)) ? 1 : 0;
 }
 
 int fa_backward_accumulate(const fa_problem_t* p, const void* q, const void* k, const void* v, const void* o,
@@ -278,7 +280,7 @@ int fa_backward_accumulate(const fa_problem_t* p, const void* q, const void* k, 
   if (!q || !k || !v || !o || !l || !m || !d_o || !dq_acc || !d_k || !d_v) return FA_EINVAL_NULL;
   const size_t need = fa_workspace_bytes(p, 1);
   if (workspace_bytes < need || (!workspace && need)) return FA_EINVAL_WORKSPACE;
-  if (p->dtype != FA_F16 || fa::g_path_override == 1 || !fa::sm100_f16_backward_accumulate_supports(a))
+  if (!is16(p->dtype) || fa::g_path_override == 1 || !fa::sm100_f16_backward_accumulate_supports(a))
     return FA_EINVAL_SHAPE;   // callers fall back to fa_backward + fa_grad_accumulate
   fa::g_last_path = 2;
   cudaError_t e = fa::sm100_f16_backward(a, (cudaStream_t)stream);
@@ -308,13 +310,14 @@ int fa_dispatch_path(const fa_problem_t* p, int is_backward, char* reason, size_
   }
   const int64_t nq = a.rule.q.total, nk = a.rule.k.total;
   const int64_t cap = 32 * int64_t(fa::sm100::kMaxTileWords);   // streamed tiles of a CTA's schedule
-  if (p->dtype == FA_F16 && (bwd ? fa::sm100_f16_backward_supports(a) : fa::sm100_f16_forward_supports(a))) return 2;
+  if (is16(p->dtype) && (bwd ? fa::sm100_f16_backward_supports(a) : fa::sm100_f16_forward_supports(a))) return 2;
   if (p->dtype == FA_F32 && (bwd ? fa::sm100_f32_backward_supports(a) : fa::sm100_f32_forward_supports(a))) return 3;
   if (p->dtype == FA_F64 && (bwd ? fa::f64_dmma_backward_supports(a) : fa::f64_dmma_forward_supports(a))) return 4;
-  const int max_ch = p->dtype == FA_F16 ? 128 : 64;
-  const int64_t tile = (p->dtype == FA_F16 && !bwd && (p->d > 64 || p->v_d > 64)) ? 128 : 64;
+  const int max_ch = is16(p->dtype) ? 128 : 64;
+  const int64_t tile = (is16(p->dtype) && !bwd && (p->d > 64 || p->v_d > 64)) ? 128 : 64;
   if (a.layout != 0) {
-    say("channel-last operands are read directly only by the fp16 tensor-core kernels (channels multiples of 8 up to 128)");
+    say("channel-last operands are read directly only by the 16-bit tensor-core kernels (channels multiples of 8 up to "
+        "128)");
     return FA_EINVAL_LAYOUT;
   }
   if (p->d > 256 || p->v_d > 256) {
@@ -327,7 +330,7 @@ int fa_dispatch_path(const fa_problem_t* p, int is_backward, char* reason, size_
     return 1;
   }
   if (p->d > max_ch || p->v_d > max_ch)
-    say(p->dtype == FA_F16 ? "more than 128 channels: generic kernels" : "more than 64 channels: generic kernels");
+    say(is16(p->dtype) ? "more than 128 channels: generic kernels" : "more than 64 channels: generic kernels");
   else if (!bwd && a.accumulate)
     say("accumulate = 1 is served by the generic forward kernels");
   else if (p->dtype != FA_F64 && ((nk + tile - 1) / tile > cap || (bwd && (nq + 63) / 64 > cap)))
@@ -341,7 +344,7 @@ int fa_dispatch_path(const fa_problem_t* p, int is_backward, char* reason, size_
 // ---- layout adapter ------------------------------------------------------------------------------
 int fa_layout_transpose(int32_t dtype, const void* x, void* y, int64_t batch, int64_t seq, int32_t heads,
                         int32_t channels, int to_channel_first, void* stream) {
-  if (dtype < FA_F16 || dtype > FA_F64) return FA_EINVAL_DTYPE;
+  if (dtype < FA_F16 || dtype > FA_BF16) return FA_EINVAL_DTYPE;
   if (batch < 0 || seq < 0 || heads < 0 || channels < 0) return FA_EINVAL_SHAPE;
   if (batch * heads > 0x7fffffffLL || (seq + 31) / 32 > 65535 || (channels + 31) / 32 > 65535) return FA_EINVAL_SHAPE;
   if (batch * seq * heads * channels == 0) return FA_OK;
@@ -352,7 +355,7 @@ int fa_layout_transpose(int32_t dtype, const void* x, void* y, int64_t batch, in
 
 // ---- gradient shards (ring backward) ---------------------------------------------------------
 int fa_grad_accumulate(int32_t dtype, const void* part, void* acc, int64_t n, int first, void* stream) {
-  if (dtype < FA_F16 || dtype > FA_F64) return FA_EINVAL_DTYPE;
+  if (dtype < FA_F16 || dtype > FA_BF16) return FA_EINVAL_DTYPE;
   if (n < 0) return FA_EINVAL_SHAPE;
   if (n == 0) return FA_OK;
   if (!part || !acc) return FA_EINVAL_NULL;
@@ -360,7 +363,7 @@ int fa_grad_accumulate(int32_t dtype, const void* part, void* acc, int64_t n, in
   return e == cudaSuccess ? FA_OK : cuda_fail(e);
 }
 int fa_grad_finalize(int32_t dtype, const void* acc, void* out, int64_t n, void* stream) {
-  if (dtype < FA_F16 || dtype > FA_F64) return FA_EINVAL_DTYPE;
+  if (dtype < FA_F16 || dtype > FA_BF16) return FA_EINVAL_DTYPE;
   if (n < 0) return FA_EINVAL_SHAPE;
   if (n == 0) return FA_OK;
   if (!acc || !out) return FA_EINVAL_NULL;

@@ -1,4 +1,6 @@
-// fa_bwd_f16_sm100.cu — Blackwell-native fp16 backward: two tcgen05/TMEM/TMA kernels.
+// fa_bwd_f16_sm100.cu — Blackwell-native 16-bit (fp16 / bf16) backward: two tcgen05/TMEM/TMA kernels.
+// Every kernel takes the element type T (__half or __nv_bfloat16) of Q, K, V, O, m, dO and the gradients, which is also
+// the type P and dS are handed to the tensor cores in.
 //
 // Replaces the reference's BackwardImpl (flash_attention/kernel/flash_attention.cu:1079-1967), which
 // keeps a K/V tile per CTA, loops over Q tiles under a global spin lock and read-modify-writes dQ in
@@ -24,6 +26,8 @@
 
 #include <cudaTypedefs.h>
 
+#include <type_traits>
+
 namespace fa {
 namespace sm100 {
 
@@ -32,9 +36,9 @@ using namespace ptx;
 bool make_map_2d(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int box_cols, int box_rows,
                  bool swizzle128);  // fa_fwd_f16_sm100.cu
 bool make_map_3d(CUtensorMap* map, const void* base, int64_t batch, int64_t channels, int64_t seq, int64_t pitch,
-                 int box_rows, bool swizzle128);  // fa_fwd_f16_sm100.cu
+                 int box_rows, bool swizzle128, CUtensorMapDataType dtype);  // fa_fwd_f16_sm100.cu
 bool make_map_cl(CUtensorMap* map, const void* base, int64_t outer, int64_t heads, int64_t channels, int64_t seq,
-                 int box_rows);  // fa_fwd_f16_sm100.cu
+                 int box_rows, CUtensorMapDataType dtype);  // fa_fwd_f16_sm100.cu
 
 // Workspace of the fp16 backward: [LSE2, D (+ pad)] [fp32 dQ scratch of the fused head_dim-128 kernel] [pitch-padded
 // copies of the q-length / k-length tensors when their length is not a multiple of 8 (fa_pack.cu)].
@@ -53,13 +57,19 @@ constexpr int kStatPad = 64;    // padding (floats) behind the LSE2 / D arrays f
 // dS enters the tensor cores as fp16. |dS| = P |dP - D| reaches several units on rows that attend few keys, where one
 // fp16 rounding (relative 2^-11) is already ~1e-3 absolute, and dK / dQ sum such terms. With SPLIT the softmax warps
 // hand over dS as a hi + lo pair of fp16 values (lo = fp16(dS - hi), written into the TMEM columns the packed hi half
-// leaves free) and the products dQ = dS K, dK = dS^T Q are issued twice, so dS carries ~22 mantissa bits.
-__device__ __forceinline__ void split_half2(float a, float b, uint32_t& hi, uint32_t& lo) {
+// leaves free) and the products dQ = dS K, dK = dS^T Q are issued twice, so dS carries ~22 mantissa bits (bf16: the
+// same pair of bf16 values, ~16 bits).
+template <typename T> __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo);
+template <> __device__ __forceinline__ void split2<__half>(float a, float b, uint32_t& hi, uint32_t& lo) {
   const __half2 h = __floats2half2_rn(a, b);
   const float2 f = __half22float2(h);
   const __half2 l = __floats2half2_rn(a - f.x, b - f.y);
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
+}
+template <> __device__ __forceinline__ void split2<__nv_bfloat16>(float a, float b, uint32_t& hi, uint32_t& lo) {
+  hi = pack2<__nv_bfloat16>(a, b);
+  lo = pack2<__nv_bfloat16>(a - __uint_as_float(hi << 16), b - __uint_as_float(hi & 0xffff0000u));
 }
 
 struct alignas(64) BwdParams {
@@ -77,8 +87,9 @@ struct alignas(64) BwdParams {
 };
 
 // ---- preprocess: LSE2 and D -------------------------------------------------------------------
-__global__ void bwd_prep_f16(const __half* __restrict__ o, const __half* __restrict__ d_o,
-                             const float* __restrict__ l, const __half* __restrict__ m, float* __restrict__ lse2,
+template <typename T>
+__global__ void bwd_prep_f16(const T* __restrict__ o, const T* __restrict__ d_o,
+                             const float* __restrict__ l, const T* __restrict__ m, float* __restrict__ lse2,
                              float* __restrict__ dsum, int64_t batch, int32_t v_d, int32_t nq, int32_t sp) {
   const int64_t total = batch * sp;
   // the padding behind both arrays (and behind each batch element's row when nq is not a multiple of 4) is read by the
@@ -88,7 +99,7 @@ __global__ void bwd_prep_f16(const __half* __restrict__ o, const __half* __restr
     lse2[total + threadIdx.x] = __int_as_float(0x7f800000);
     dsum[total + threadIdx.x] = 0.f;
   }
-  // two adjacent query positions per thread -> half2 loads, coalesced along the sequence (nq and sp are even here)
+  // two adjacent query positions per thread -> pair loads, coalesced along the sequence (nq and sp are even here)
   for (int64_t i2 = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) * 2; i2 < total;
        i2 += int64_t(gridDim.x) * blockDim.x * 2) {
     const int64_t b = i2 / sp, r = i2 - b * sp;
@@ -97,14 +108,14 @@ __global__ void bwd_prep_f16(const __half* __restrict__ o, const __half* __restr
       dsum[i2] = dsum[i2 + 1] = 0.f;
       continue;
     }
-    const __half2* op = reinterpret_cast<const __half2*>(o + b * v_d * int64_t(nq) + r);
-    const __half2* dp = reinterpret_cast<const __half2*>(d_o + b * v_d * int64_t(nq) + r);
+    const Pair<T>* op = reinterpret_cast<const Pair<T>*>(o + b * v_d * int64_t(nq) + r);
+    const Pair<T>* dp = reinterpret_cast<const Pair<T>*>(d_o + b * v_d * int64_t(nq) + r);
     float a0 = 0.f, a1 = 0.f;
     const int64_t pitch2 = nq / 2;
 #pragma unroll 4
     for (int c = 0; c < v_d; ++c) {
-      const float2 x = __half22float2(op[c * pitch2]);
-      const float2 y = __half22float2(dp[c * pitch2]);
+      const float2 x = to_float2(op[c * pitch2]);
+      const float2 y = to_float2(dp[c * pitch2]);
       a0 = fmaf(x.x, y.x, a0);
       a1 = fmaf(x.y, y.y, a1);
     }
@@ -113,16 +124,17 @@ __global__ void bwd_prep_f16(const __half* __restrict__ o, const __half* __restr
 #pragma unroll
     for (int e = 0; e < 2; ++e) {
       const float lv = l[b * nq + r + e];
-      const __half mv = m[b * nq + r + e];
-      lse2[i2 + e] = (lv > 0.f && !is_sentinel<__half>(mv)) ? (__half2float(mv) + logf(lv)) * kLog2eB
+      const T mv = m[b * nq + r + e];
+      lse2[i2 + e] = (lv > 0.f && !is_sentinel<T>(mv)) ? (to_acc<float>(mv) + logf(lv)) * kLog2eB
                                                              : __int_as_float(0x7f800000);
     }
   }
 }
 
 // any query length (odd included): one thread per query position, scalar loads coalesced along the sequence
-__global__ void bwd_prep_f16_any(const __half* __restrict__ o, const __half* __restrict__ d_o,
-                                 const float* __restrict__ l, const __half* __restrict__ m, float* __restrict__ lse2,
+template <typename T>
+__global__ void bwd_prep_f16_any(const T* __restrict__ o, const T* __restrict__ d_o,
+                                 const float* __restrict__ l, const T* __restrict__ m, float* __restrict__ lse2,
                                  float* __restrict__ dsum, int64_t batch, int32_t v_d, int32_t nq, int32_t sp) {
   const int64_t total = batch * sp;
   if (blockIdx.x == gridDim.x - 1 && threadIdx.x < kStatPad) {
@@ -136,15 +148,15 @@ __global__ void bwd_prep_f16_any(const __half* __restrict__ o, const __half* __r
       dsum[i] = 0.f;
       continue;
     }
-    const __half* op = o + b * v_d * int64_t(nq) + r;
-    const __half* dp = d_o + b * v_d * int64_t(nq) + r;
+    const T* op = o + b * v_d * int64_t(nq) + r;
+    const T* dp = d_o + b * v_d * int64_t(nq) + r;
     float acc = 0.f;
 #pragma unroll 4
-    for (int c = 0; c < v_d; ++c) acc = fmaf(__half2float(op[c * int64_t(nq)]), __half2float(dp[c * int64_t(nq)]), acc);
+    for (int c = 0; c < v_d; ++c) acc = fmaf(to_acc<float>(op[c * int64_t(nq)]), to_acc<float>(dp[c * int64_t(nq)]), acc);
     dsum[i] = acc;
     const float lv = l[b * nq + r];
-    const __half mv = m[b * nq + r];
-    lse2[i] = (lv > 0.f && !is_sentinel<__half>(mv)) ? (__half2float(mv) + logf(lv)) * kLog2eB
+    const T mv = m[b * nq + r];
+    lse2[i] = (lv > 0.f && !is_sentinel<T>(mv)) ? (to_acc<float>(mv) + logf(lv)) * kLog2eB
                                                       : __int_as_float(0x7f800000);
   }
 }
@@ -152,9 +164,9 @@ __global__ void bwd_prep_f16_any(const __half* __restrict__ o, const __half* __r
 // channel-last O / dO ([outer][q][heads][v_d], v_d a multiple of 8): a group of G lanes (the power of two >= v_d / 8)
 // reads one row's channels as 16-byte chunks and reduces with shuffles; one thread per (outer, q, head) row would touch
 // 16 bytes of every 2 * v_d-byte row per instruction
-template <int G>
-__global__ void bwd_prep_f16_cl(const __half* __restrict__ o, const __half* __restrict__ d_o,
-                                const float* __restrict__ l, const __half* __restrict__ m, float* __restrict__ lse2,
+template <typename T, int G>
+__global__ void bwd_prep_f16_cl(const T* __restrict__ o, const T* __restrict__ d_o,
+                                const float* __restrict__ l, const T* __restrict__ m, float* __restrict__ lse2,
                                 float* __restrict__ dsum, int64_t outer, int32_t heads, int32_t v_d, int32_t nq,
                                 int32_t sp) {
   const int64_t batch = outer * heads, total = batch * sp;
@@ -182,11 +194,11 @@ __global__ void bwd_prep_f16_cl(const __half* __restrict__ o, const __half* __re
     if (live && g * 8 < v_d) {
       const uint4 x = *reinterpret_cast<const uint4*>(o + row * v_d + g * 8);
       const uint4 y = *reinterpret_cast<const uint4*>(d_o + row * v_d + g * 8);
-      const __half2* xh = reinterpret_cast<const __half2*>(&x);
-      const __half2* yh = reinterpret_cast<const __half2*>(&y);
+      const Pair<T>* xh = reinterpret_cast<const Pair<T>*>(&x);
+      const Pair<T>* yh = reinterpret_cast<const Pair<T>*>(&y);
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
-        const float2 a = __half22float2(xh[e]), c = __half22float2(yh[e]);
+        const float2 a = to_float2(xh[e]), c = to_float2(yh[e]);
         acc = fmaf(a.x, c.x, acc);
         acc = fmaf(a.y, c.y, acc);
       }
@@ -198,8 +210,8 @@ __global__ void bwd_prep_f16_cl(const __half* __restrict__ o, const __half* __re
       const int64_t b = ob * heads + h;
       dsum[b * sp + q] = acc;
       const float lv = l[b * nq + q];
-      const __half mv = m[b * nq + q];
-      lse2[b * sp + q] = (lv > 0.f && !is_sentinel<__half>(mv)) ? (__half2float(mv) + logf(lv)) * kLog2eB
+      const T mv = m[b * nq + q];
+      lse2[b * sp + q] = (lv > 0.f && !is_sentinel<T>(mv)) ? (to_acc<float>(mv) + logf(lv)) * kLog2eB
                                                                  : __int_as_float(0x7f800000);
     }
   }
@@ -223,7 +235,7 @@ struct DqCfg {
   static constexpr int kSmemBytes = kSchedOffset + int(sizeof(TileSchedule)) + 1024;
 };
 
-template <int D, int VD, bool SPLIT, bool CL>
+template <typename T, int D, int VD, bool SPLIT, bool CL>
 __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dq_kernel(const __grid_constant__ BwdParams p) {
   using Cfg = DqCfg<D, VD>;
   constexpr int kStages = Cfg::kStages;
@@ -323,8 +335,8 @@ __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dq_kernel(const __grid_con
         TileIter it;
         it.init(sched, 2, kt_first, kt_last);
         const int n = it.count();
-        constexpr uint32_t idesc_s = idesc_f16(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
-        constexpr uint32_t idesc_dq = idesc_f16(kBM, D, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_s = idesc_16<T>(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
+        constexpr uint32_t idesc_dq = idesc_16<T>(kBM, D, false, tile_mn_major<CL>(false));
         auto issue_s_dp = [&](int i, int stage) {
           const uint32_t k_s = ring + stage * Cfg::kStageBytes, v_s = k_s + Cfg::kKBytes;
 #pragma unroll
@@ -448,12 +460,12 @@ __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dq_kernel(const __grid_con
         if constexpr (kExact) {
           d_exact = fmaf(p0, dp[c], d_exact);
           d_exact = fmaf(p1, dp[c + 1], d_exact);
-          pp[c >> 1] = pack_half2(p0, p1);
+          pp[c >> 1] = pack2<T>(p0, p1);
         }
         if constexpr (SPLIT)
-          split_half2(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum), pk[c >> 1], pl[c >> 1]);
+          split2<T>(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum), pk[c >> 1], pl[c >> 1]);
         else
-          pk[c >> 1] = pack_half2(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum));
+          pk[c >> 1] = pack2<T>(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum));
       }
       tmem_st32(t_s, pk);
       if constexpr (SPLIT) tmem_st32(t_s + 32, pl);
@@ -487,7 +499,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dq_kernel(const __grid_con
 #pragma unroll
           for (int e = 0; e < 32; ++e) o[e] = fmaf(-delta, o2[e], o[e]);
         }
-        stage_row32<CL>(stage_gen, r, c * 32, kBM, D, o, p.scale);
+        stage_row32<CL, T>(stage_gen, r, c * 32, kBM, D, o, p.scale);
       }
     } else {
       mbar_wait(bar_q_full + 8 * i, 0);
@@ -528,7 +540,7 @@ struct DqSmallCfg {
   static constexpr int kSmemBytes = kSchedOffset + int(sizeof(TileSchedule)) + 1024;
 };
 
-template <int D, int VD, bool SPLIT, bool CL>
+template <typename T, int D, int VD, bool SPLIT, bool CL>
 __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dq_small_kernel(const __grid_constant__ BwdParams p) {
   using Cfg = DqSmallCfg<D, VD>;
   constexpr int kStages = Cfg::kStages;
@@ -629,8 +641,8 @@ __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dq_small_kernel(const __gr
         TileIter it;
         it.init(sched, 1, kt_first, kt_last);
         const int n = it.count();
-        constexpr uint32_t idesc_s = idesc_f16(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
-        constexpr uint32_t idesc_dq = idesc_f16(kBM, D, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_s = idesc_16<T>(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
+        constexpr uint32_t idesc_dq = idesc_16<T>(kBM, D, false, tile_mn_major<CL>(false));
         auto issue_s_dp = [&](int stage) {
           const uint32_t k_s = ring + stage * Cfg::kStageBytes, v_s = k_s + Cfg::kKBytes;
 #pragma unroll
@@ -735,10 +747,10 @@ __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dq_small_kernel(const __gr
         if constexpr (SPLIT) {
           d_exact = fmaf(p0, dp[c], d_exact);
           d_exact = fmaf(p1, dp[c + 1], d_exact);
-          split_half2(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum), pk[c >> 1], pl[c >> 1]);
-          pp[c >> 1] = pack_half2(p0, p1);
+          split2<T>(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum), pk[c >> 1], pl[c >> 1]);
+          pp[c >> 1] = pack2<T>(p0, p1);
         } else {
-          pk[c >> 1] = pack_half2(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum));
+          pk[c >> 1] = pack2<T>(p0 * (dp[c] - dsum), p1 * (dp[c + 1] - dsum));
         }
       }
       tmem_st16(t_s, pk);
@@ -779,7 +791,7 @@ __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dq_small_kernel(const __gr
 #pragma unroll
           for (int e = 0; e < 32; ++e) o[e] = fmaf(-delta, o2[e], o[e]);
         }
-        stage_row32<CL>(stage_gen, r, c * 32, kBM, D, o, p.scale);
+        stage_row32<CL, T>(stage_gen, r, c * 32, kBM, D, o, p.scale);
       }
     } else {
       mbar_wait(bar_q_full, 0);
@@ -829,7 +841,7 @@ __device__ __forceinline__ void bulk_load_1d(uint32_t smem_dst, const void* gsrc
                : "memory");
 }
 
-template <int D, int VD, bool SPLIT, bool CL>
+template <typename T, int D, int VD, bool SPLIT, bool CL>
 __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dkdv_kernel(const __grid_constant__ BwdParams p) {
   using Cfg = DkvCfg<D, VD>;
   constexpr int kStages = Cfg::kStages;
@@ -930,9 +942,9 @@ __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dkdv_kernel(const __grid_c
         TileIter it;
         it.init(sched, 1, qt_first, qt_last);
         const int n = it.count();
-        constexpr uint32_t idesc_st = idesc_f16(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
-        constexpr uint32_t idesc_dv = idesc_f16(kBM, VD, false, tile_mn_major<CL>(false));
-        constexpr uint32_t idesc_dk = idesc_f16(kBM, D, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_st = idesc_16<T>(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
+        constexpr uint32_t idesc_dv = idesc_16<T>(kBM, VD, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_dk = idesc_16<T>(kBM, D, false, tile_mn_major<CL>(false));
         auto issue_st_dpt = [&](int x, int stage) {
           const uint32_t q_s = ring + stage * Cfg::kStageBytes, do_s = q_s + Cfg::kQBytes;
 #pragma unroll
@@ -1055,13 +1067,13 @@ __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dkdv_kernel(const __grid_c
         p0 = (mword >> (c & 31)) & 1u ? p0 : 0.f;
         p1 = (mword >> ((c + 1) & 31)) & 1u ? p1 : 0.f;
         if constexpr (SPLIT)
-          split_half2(p0, p1, pk[c >> 1], pl[c >> 1]);
+          split2<T>(p0, p1, pk[c >> 1], pl[c >> 1]);
         else
-          pk[c >> 1] = pack_half2(p0, p1);
+          pk[c >> 1] = pack2<T>(p0, p1);
         if constexpr (SPLIT)
-          split_half2(p0 * (dp[c] - dsum_s[c]), p1 * (dp[c + 1] - dsum_s[c + 1]), dk[c >> 1], dl[c >> 1]);
+          split2<T>(p0 * (dp[c] - dsum_s[c]), p1 * (dp[c + 1] - dsum_s[c + 1]), dk[c >> 1], dl[c >> 1]);
         else
-          dk[c >> 1] = pack_half2(p0 * (dp[c] - dsum_s[c]), p1 * (dp[c + 1] - dsum_s[c + 1]));
+          dk[c >> 1] = pack2<T>(p0 * (dp[c] - dsum_s[c]), p1 * (dp[c + 1] - dsum_s[c + 1]));
       }
       tmem_st32(t_s, pk);
       tmem_st32(t_dp, dk);
@@ -1087,7 +1099,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) bwd_dkdv_kernel(const __grid_c
         float o[32];
         tmem_ld32f(t_acc + c * 32, o);
         tmem_wait_ld();
-        stage_row32<CL>(stage_gen, r, c * 32, kBM, CH, o, out_scale);
+        stage_row32<CL, T>(stage_gen, r, c * 32, kBM, CH, o, out_scale);
       }
     } else {
       mbar_wait(bar_kv_res, 0);
@@ -1133,7 +1145,7 @@ struct DkvSmallCfg {
   static constexpr int kSmemBytes = kSchedOffset + int(sizeof(TileSchedule)) + 1024;
 };
 
-template <int D, int VD, bool SPLIT, bool CL>
+template <typename T, int D, int VD, bool SPLIT, bool CL>
 __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dkdv_small_kernel(const __grid_constant__ BwdParams p) {
   using Cfg = DkvSmallCfg<D, VD>;
   constexpr int kStages = Cfg::kStages;
@@ -1236,9 +1248,9 @@ __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dkdv_small_kernel(const __
         TileIter it;
         it.init(sched, 1, qt_first, qt_last);
         const int n = it.count();
-        constexpr uint32_t idesc_st = idesc_f16(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
-        constexpr uint32_t idesc_dv = idesc_f16(kBM, VD, false, tile_mn_major<CL>(false));
-        constexpr uint32_t idesc_dk = idesc_f16(kBM, D, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_st = idesc_16<T>(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
+        constexpr uint32_t idesc_dv = idesc_16<T>(kBM, VD, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_dk = idesc_16<T>(kBM, D, false, tile_mn_major<CL>(false));
         auto issue_st_dpt = [&](int stage) {
           const uint32_t q_s = ring + stage * Cfg::kStageBytes, do_s = q_s + Cfg::kQBytes;
 #pragma unroll
@@ -1357,18 +1369,18 @@ __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dkdv_small_kernel(const __
         p2 = mword & 4u ? p2 : 0.f;
         p3 = mword & 8u ? p3 : 0.f;
         if constexpr (SPLIT) {
-          split_half2(p0, p1, pk[c >> 1], pl[c >> 1]);
-          split_half2(p2, p3, pk[(c >> 1) + 1], pl[(c >> 1) + 1]);
+          split2<T>(p0, p1, pk[c >> 1], pl[c >> 1]);
+          split2<T>(p2, p3, pk[(c >> 1) + 1], pl[(c >> 1) + 1]);
         } else {
-          pk[c >> 1] = pack_half2(p0, p1);
-          pk[(c >> 1) + 1] = pack_half2(p2, p3);
+          pk[c >> 1] = pack2<T>(p0, p1);
+          pk[(c >> 1) + 1] = pack2<T>(p2, p3);
         }
         if constexpr (SPLIT) {
-          split_half2(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y), dk[c >> 1], dl[c >> 1]);
-          split_half2(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w), dk[(c >> 1) + 1], dl[(c >> 1) + 1]);
+          split2<T>(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y), dk[c >> 1], dl[c >> 1]);
+          split2<T>(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w), dk[(c >> 1) + 1], dl[(c >> 1) + 1]);
         } else {
-          dk[c >> 1] = pack_half2(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y));
-          dk[(c >> 1) + 1] = pack_half2(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w));
+          dk[c >> 1] = pack2<T>(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y));
+          dk[(c >> 1) + 1] = pack2<T>(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w));
         }
       }
       tmem_st16(t_s, pk);          // P^T  over the first 16 columns of this half of S^T
@@ -1395,7 +1407,7 @@ __global__ void __launch_bounds__(kBwdThreads, 2) bwd_dkdv_small_kernel(const __
         float o[32];
         tmem_ld32f(t_acc + c * 32, o);
         tmem_wait_ld();
-        stage_row32<CL>(stage_gen, r, c * 32, kBM, CH, o, out_scale);
+        stage_row32<CL, T>(stage_gen, r, c * 32, kBM, CH, o, out_scale);
       }
     } else {
       mbar_wait(bar_kv_res, 0);
@@ -1507,7 +1519,7 @@ struct alignas(64) FusedParams {
   int32_t dq_fold;
 };
 
-template <int D, int VD, bool CL, bool ACC>
+template <typename T, int D, int VD, bool CL, bool ACC>
 __global__ void __launch_bounds__(kFusedThreads, 1) bwd_fused_kernel(const __grid_constant__ FusedParams fp) {
   using Cfg = FusedCfg<D, VD>;
   constexpr int kStages = Cfg::kStages;
@@ -1677,10 +1689,10 @@ __global__ void __launch_bounds__(kFusedThreads, 1) bwd_fused_kernel(const __gri
         TileIter it;
         it.init(sched, 1, qt_first, qt_last);
         const int n = it.count();
-        constexpr uint32_t idesc_st = idesc_f16(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
-        constexpr uint32_t idesc_dv = idesc_f16(kBM, VD, false, tile_mn_major<CL>(false));
-        constexpr uint32_t idesc_dk = idesc_f16(kBM, D, false, tile_mn_major<CL>(false));
-        constexpr uint32_t idesc_dq = idesc_f16(D, kBN, tile_mn_major<CL>(false), true);
+        constexpr uint32_t idesc_st = idesc_16<T>(kBM, kBN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
+        constexpr uint32_t idesc_dv = idesc_16<T>(kBM, VD, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_dk = idesc_16<T>(kBM, D, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_dq = idesc_16<T>(D, kBN, tile_mn_major<CL>(false), true);
         auto issue_st = [&](int x, int stage) {
           const uint32_t q_s = ring + stage * Cfg::kStageBytes;
 #pragma unroll
@@ -1815,10 +1827,10 @@ __global__ void __launch_bounds__(kFusedThreads, 1) bwd_fused_kernel(const __gri
           const float p1 = ex2(fmaf(s[c + 1], scale_log2, -ls.y));
           const float p2 = ex2(fmaf(s[c + 2], scale_log2, -ls.z));
           const float p3 = ex2(fmaf(s[c + 3], scale_log2, -ls.w));
-          pk[c >> 1] = pack_half2(p0, p1);
-          pk[(c >> 1) + 1] = pack_half2(p2, p3);
-          dk[c >> 1] = pack_half2(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y));
-          dk[(c >> 1) + 1] = pack_half2(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w));
+          pk[c >> 1] = pack2<T>(p0, p1);
+          pk[(c >> 1) + 1] = pack2<T>(p2, p3);
+          dk[c >> 1] = pack2<T>(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y));
+          dk[(c >> 1) + 1] = pack2<T>(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w));
         }
       } else {
 #pragma unroll
@@ -1834,10 +1846,10 @@ __global__ void __launch_bounds__(kFusedThreads, 1) bwd_fused_kernel(const __gri
           p1 = mword & 2u ? p1 : 0.f;
           p2 = mword & 4u ? p2 : 0.f;
           p3 = mword & 8u ? p3 : 0.f;
-          pk[c >> 1] = pack_half2(p0, p1);
-          pk[(c >> 1) + 1] = pack_half2(p2, p3);
-          dk[c >> 1] = pack_half2(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y));
-          dk[(c >> 1) + 1] = pack_half2(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w));
+          pk[c >> 1] = pack2<T>(p0, p1);
+          pk[(c >> 1) + 1] = pack2<T>(p2, p3);
+          dk[c >> 1] = pack2<T>(p0 * (dp[c] - dd.x), p1 * (dp[c + 1] - dd.y));
+          dk[(c >> 1) + 1] = pack2<T>(p2 * (dp[c + 2] - dd.z), p3 * (dp[c + 3] - dd.w));
         }
       }
       if (r == 0) FB_STAMP(0, t, 2);
@@ -1867,7 +1879,7 @@ __global__ void __launch_bounds__(kFusedThreads, 1) bwd_fused_kernel(const __gri
           float o[32];
           tmem_ld32f(t_acc + c * 32, o);
           tmem_wait_ld();
-          stage_row32<CL>(stage_gen, r, c * 32, kBM, CH, o, out_scale);
+          stage_row32<CL, T>(stage_gen, r, c * 32, kBM, CH, o, out_scale);
         }
       } else {
         mbar_wait(bar_kv_res, 0);
@@ -1893,27 +1905,29 @@ __global__ void __launch_bounds__(kFusedThreads, 1) bwd_fused_kernel(const __gri
   }
 }
 
-// dQ = fp16(scale * dQ_acc); 8 elements per thread
+// dQ = T(scale * dQ_acc); 8 elements per thread
+template <typename T>
 __global__ void bwd_dq_convert(const float4* __restrict__ acc, uint4* __restrict__ dq, int64_t n8, float scale) {
   for (int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; i < n8; i += int64_t(gridDim.x) * blockDim.x) {
     const float4 a = acc[2 * i], c = acc[2 * i + 1];
     uint4 o;
-    o.x = pack_half2(a.x * scale, a.y * scale);
-    o.y = pack_half2(a.z * scale, a.w * scale);
-    o.z = pack_half2(c.x * scale, c.y * scale);
-    o.w = pack_half2(c.z * scale, c.w * scale);
+    o.x = pack2<T>(a.x * scale, a.y * scale);
+    o.y = pack2<T>(a.z * scale, a.w * scale);
+    o.z = pack2<T>(c.x * scale, c.y * scale);
+    o.w = pack2<T>(c.z * scale, c.w * scale);
     dq[i] = o;
   }
 }
 
 // channel-last dQ: the fused kernel's scratch stays [batch * 128][pitch] fp32 (its drain is layout-independent); this
 // pass scales, rounds and transposes 64 positions x 128 channels per block through shared memory into
-// [outer][q][heads][128] fp16
-__global__ void __launch_bounds__(256) bwd_dq_convert_cl(const float* __restrict__ acc, __half* __restrict__ dq,
+// [outer][q][heads][128] T
+template <typename T>
+__global__ void __launch_bounds__(256) bwd_dq_convert_cl(const float* __restrict__ acc, T* __restrict__ dq,
                                                          int64_t batch, int32_t nq, int64_t pitch, int32_t heads,
                                                          float scale) {
   constexpr int kPitch = 130;   // halves per staged position row: 4-byte aligned rows, 2-way bank conflicts at most
-  __shared__ __half tile[64 * kPitch];
+  __shared__ T tile[64 * kPitch];
   const int q0 = blockIdx.x * 64;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int q = q0 + 2 * lane;
@@ -1921,14 +1935,14 @@ __global__ void __launch_bounds__(256) bwd_dq_convert_cl(const float* __restrict
     for (int d = warp; d < 128; d += 8) {
       float2 v = make_float2(0.f, 0.f);
       if (q < pitch) v = *reinterpret_cast<const float2*>(acc + (b * 128 + d) * pitch + q);   // pitch is even
-      tile[(2 * lane) * kPitch + d] = __float2half_rn(v.x * scale);
-      tile[(2 * lane + 1) * kPitch + d] = __float2half_rn(v.y * scale);
+      tile[(2 * lane) * kPitch + d] = from_acc<T>(v.x * scale);
+      tile[(2 * lane + 1) * kPitch + d] = from_acc<T>(v.y * scale);
     }
     __syncthreads();
     const int64_t ob = b / heads, h = b % heads;
     for (int r = warp; r < 64 && q0 + r < nq; r += 8) {
-      __half2* dst = reinterpret_cast<__half2*>(dq + ((ob * nq + q0 + r) * heads + h) * 128);
-      const __half2* src = reinterpret_cast<const __half2*>(tile + r * kPitch);
+      Pair<T>* dst = reinterpret_cast<Pair<T>*>(dq + ((ob * nq + q0 + r) * heads + h) * 128);
+      const Pair<T>* src = reinterpret_cast<const Pair<T>*>(tile + r * kPitch);
       dst[lane] = src[lane];
       dst[lane + 32] = src[lane + 32];
     }
@@ -1965,32 +1979,34 @@ static bool precise_auto(const FaRule& r) {
 // Tensor maps of one kernel. Channel-first boxes are 64 positions x the kernel's channels for every kernel; a
 // channel-last box is 64 channels x the tile's rows, which differ per kernel: rq rows for the q-length tensors
 // (Q, dO, dQ), rk for the k-length ones.
-template <int D, int VD, bool CL>
+template <typename T, int D, int VD, bool CL>
 static bool bwd_maps(BwdParams* p, const LaunchArgs& a, int rq, int rk) {
   const int nq = a.rule.q.total, nk = a.rule.k.total;
+  constexpr CUtensorMapDataType dt = Elt16<T>::kTmaType;
   if constexpr (CL) {
     const int64_t heads = a.heads, outer = a.batch / heads;
-    return make_map_cl(&p->map_q, a.q, outer, heads, a.d, nq, rq) && make_map_cl(&p->map_k, a.k, outer, heads, a.d, nk, rk) &&
-           make_map_cl(&p->map_v, a.v, outer, heads, a.v_d, nk, rk) &&
-           make_map_cl(&p->map_do, a.d_o, outer, heads, a.v_d, nq, rq) &&
-           make_map_cl(&p->map_dq, a.d_q, outer, heads, a.d, nq, rq) &&
-           make_map_cl(&p->map_dk, a.d_k, outer, heads, a.d, nk, rk) &&
-           make_map_cl(&p->map_dv, a.d_v, outer, heads, a.v_d, nk, rk);
+    return make_map_cl(&p->map_q, a.q, outer, heads, a.d, nq, rq, dt) && make_map_cl(&p->map_k, a.k, outer, heads, a.d, nk, rk, dt) &&
+           make_map_cl(&p->map_v, a.v, outer, heads, a.v_d, nk, rk, dt) &&
+           make_map_cl(&p->map_do, a.d_o, outer, heads, a.v_d, nq, rq, dt) &&
+           make_map_cl(&p->map_dq, a.d_q, outer, heads, a.d, nq, rq, dt) &&
+           make_map_cl(&p->map_dk, a.d_k, outer, heads, a.d, nk, rk, dt) &&
+           make_map_cl(&p->map_dv, a.d_v, outer, heads, a.v_d, nk, rk, dt);
   } else {
     const int64_t qp = a.q_pitch ? a.q_pitch : nq, kp = a.k_pitch ? a.k_pitch : nk;
-    return make_map_3d(&p->map_q, a.q, a.batch, a.d, nq, qp, D, true) &&
-           make_map_3d(&p->map_k, a.k, a.batch, a.d, nk, kp, D, true) &&
-           make_map_3d(&p->map_v, a.v, a.batch, a.v_d, nk, kp, VD, true) &&
-           make_map_3d(&p->map_do, a.d_o, a.batch, a.v_d, nq, qp, VD, true) &&
-           make_map_3d(&p->map_dq, a.d_q, a.batch, a.d, nq, qp, D, false) &&
-           make_map_3d(&p->map_dk, a.d_k, a.batch, a.d, nk, kp, D, false) &&
-           make_map_3d(&p->map_dv, a.d_v, a.batch, a.v_d, nk, kp, VD, false);
+    return make_map_3d(&p->map_q, a.q, a.batch, a.d, nq, qp, D, true, dt) &&
+           make_map_3d(&p->map_k, a.k, a.batch, a.d, nk, kp, D, true, dt) &&
+           make_map_3d(&p->map_v, a.v, a.batch, a.v_d, nk, kp, VD, true, dt) &&
+           make_map_3d(&p->map_do, a.d_o, a.batch, a.v_d, nq, qp, VD, true, dt) &&
+           make_map_3d(&p->map_dq, a.d_q, a.batch, a.d, nq, qp, D, false, dt) &&
+           make_map_3d(&p->map_dk, a.d_k, a.batch, a.d, nk, kp, D, false, dt) &&
+           make_map_3d(&p->map_dv, a.d_v, a.batch, a.v_d, nk, kp, VD, false, dt);
   }
 }
 
 // D, VD: the kernels' padded channel counts (a.d <= D, a.v_d <= VD; the tensor maps zero-fill / clip the rest)
-template <int D, int VD, bool CL>
+template <typename T, int D, int VD, bool CL>
 cudaError_t launch_bwd(const LaunchArgs& a, cudaStream_t stream) {
+  constexpr bool kBf16 = std::is_same<T, __nv_bfloat16>::value;
   BwdParams p;
   const int nq = a.rule.q.total, nk = a.rule.k.total;
   // row pitch of the fused kernel's fp32 dQ scratch (and, channel-first, of the dQ tensor the convert pass writes)
@@ -2019,30 +2035,30 @@ cudaError_t launch_bwd(const LaunchArgs& a, cudaStream_t stream) {
   {
     // statistics from the caller's own (dense) O and dO
     const int64_t total = a.batch * sp;
-    ScopedKernel timed(CL ? "bwd_prep_f16_cl" : "bwd_prep_f16", stream);
+    ScopedKernel timed(CL ? (kBf16 ? "bwd_prep_bf16_cl" : "bwd_prep_f16_cl") : (kBf16 ? "bwd_prep_bf16" : "bwd_prep_f16"), stream);
     if constexpr (CL) {
       const int64_t outer = a.batch / a.heads;
       const int chunks = a.v_d / 8;
       const int64_t rows = outer * nq * int64_t(a.heads);
       auto go = [&](auto kern, int G) {
         const int blocks = int(std::min<int64_t>((rows * G + 255) / 256, 148 * 16));
-        kern<<<std::max(blocks, 1), 256, 0, stream>>>((const __half*)a.o, (const __half*)a.prep_d_o, (const float*)a.l,
-                                                     (const __half*)a.m, lse2, dsum, outer, a.heads, a.v_d, nq, int32_t(sp));
+        kern<<<std::max(blocks, 1), 256, 0, stream>>>((const T*)a.o, (const T*)a.prep_d_o, (const float*)a.l,
+                                                     (const T*)a.m, lse2, dsum, outer, a.heads, a.v_d, nq, int32_t(sp));
       };
-      if (chunks <= 1) go(bwd_prep_f16_cl<1>, 1);
-      else if (chunks <= 2) go(bwd_prep_f16_cl<2>, 2);
-      else if (chunks <= 4) go(bwd_prep_f16_cl<4>, 4);
-      else if (chunks <= 8) go(bwd_prep_f16_cl<8>, 8);
-      else go(bwd_prep_f16_cl<16>, 16);
+      if (chunks <= 1) go(bwd_prep_f16_cl<T, 1>, 1);
+      else if (chunks <= 2) go(bwd_prep_f16_cl<T, 2>, 2);
+      else if (chunks <= 4) go(bwd_prep_f16_cl<T, 4>, 4);
+      else if (chunks <= 8) go(bwd_prep_f16_cl<T, 8>, 8);
+      else go(bwd_prep_f16_cl<T, 16>, 16);
     } else if (nq % 2 == 0 && (reinterpret_cast<uintptr_t>(a.o) & 3) == 0 &&
                (reinterpret_cast<uintptr_t>(a.prep_d_o) & 3) == 0) {
       const int blocks = int(std::min<int64_t>((total / 2 + 255) / 256, 148 * 16));
-      bwd_prep_f16<<<blocks, 256, 0, stream>>>((const __half*)a.o, (const __half*)a.prep_d_o, (const float*)a.l,
-                                               (const __half*)a.m, lse2, dsum, a.batch, a.v_d, nq, int32_t(sp));
+      bwd_prep_f16<T><<<blocks, 256, 0, stream>>>((const T*)a.o, (const T*)a.prep_d_o, (const float*)a.l,
+                                               (const T*)a.m, lse2, dsum, a.batch, a.v_d, nq, int32_t(sp));
     } else {
       const int blocks = int(std::min<int64_t>((total + 255) / 256, 148 * 16));
-      bwd_prep_f16_any<<<blocks, 256, 0, stream>>>((const __half*)a.o, (const __half*)a.prep_d_o, (const float*)a.l,
-                                                   (const __half*)a.m, lse2, dsum, a.batch, a.v_d, nq, int32_t(sp));
+      bwd_prep_f16_any<T><<<blocks, 256, 0, stream>>>((const T*)a.o, (const T*)a.prep_d_o, (const float*)a.l,
+                                                   (const T*)a.m, lse2, dsum, a.batch, a.v_d, nq, int32_t(sp));
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
@@ -2051,7 +2067,7 @@ cudaError_t launch_bwd(const LaunchArgs& a, cudaStream_t stream) {
     if (a.variant != 4 && !split && fused_shape) {
       // fused dQ/dK/dV: fp32 dQ scratch behind the row statistics, with the row pitch of the dQ tensor the convert pass
       // writes (the padded pitch when the q side is packed; the columns past nq only ever receive zeros)
-      if (!bwd_maps<D, VD, CL>(&p, a, kBN, kBM)) return cudaErrorInvalidValue;
+      if (!bwd_maps<T, D, VD, CL>(&p, a, kBN, kBM)) return cudaErrorInvalidValue;
       if constexpr (!CL) {
         if (a.grad_acc) {
           // dQ added into the caller's fp32 accumulator through the kernel's own reduce-add: no scratch, no memset, no
@@ -2060,11 +2076,11 @@ cudaError_t launch_bwd(const LaunchArgs& a, cudaStream_t stream) {
           fp.base = p;
           fp.dq_fold = int32_t(a.dq_fold);
           if (!make_map_f32_sw128(&fp.map_dq_acc, a.d_q, a.dq_fold * D, nq, 32, D)) return cudaErrorInvalidValue;
-          auto kern = bwd_fused_kernel<D, VD, false, true>;
+          auto kern = bwd_fused_kernel<T, D, VD, false, true>;
           cudaError_t e = plan::ensure_smem(kern, FusedCfg<D, VD>::kSmemBytes);
           if (e != cudaSuccess) return e;
           fp.base.n_blocks = (nk + kBM - 1) / kBM;
-          ScopedKernel timed("bwd_fused_f16_sm100_acc", stream);
+          ScopedKernel timed((kBf16 ? "bwd_fused_bf16_sm100_acc" : "bwd_fused_f16_sm100_acc"), stream);
           kern<<<unsigned(int64_t(fp.base.n_blocks) * p.batch), kFusedThreads, FusedCfg<D, VD>::kSmemBytes, stream>>>(fp);
           return cudaGetLastError();
         }
@@ -2081,42 +2097,42 @@ cudaError_t launch_bwd(const LaunchArgs& a, cudaStream_t stream) {
         if (e != cudaSuccess) return e;
       }
       {
-        auto kern = bwd_fused_kernel<D, VD, CL, false>;
+        auto kern = bwd_fused_kernel<T, D, VD, CL, false>;
         cudaError_t e =
             plan::ensure_smem(kern, FusedCfg<D, VD>::kSmemBytes);
         if (e != cudaSuccess) return e;
         fp.base.n_blocks = (nk + kBM - 1) / kBM;
-        ScopedKernel timed(CL ? "bwd_fused_f16_sm100_cl" : "bwd_fused_f16_sm100", stream);
+        ScopedKernel timed(CL ? (kBf16 ? "bwd_fused_bf16_sm100_cl" : "bwd_fused_f16_sm100_cl") : (kBf16 ? "bwd_fused_bf16_sm100" : "bwd_fused_f16_sm100"), stream);
         kern<<<unsigned(int64_t(fp.base.n_blocks) * p.batch), kFusedThreads, FusedCfg<D, VD>::kSmemBytes, stream>>>(fp);
         e = cudaGetLastError();
         if (e != cudaSuccess) return e;
       }
       if constexpr (CL) {
-        ScopedKernel timed("bwd_dq_convert_cl", stream);
-        bwd_dq_convert_cl<<<dim3(unsigned((nq + 63) / 64), unsigned(std::min<int64_t>(a.batch, 65535))), 256, 0, stream>>>(
-            acc, reinterpret_cast<__half*>(a.d_q), a.batch, nq, qp, a.heads, p.scale);
+        ScopedKernel timed((kBf16 ? "bwd_dq_convert_bf16_cl" : "bwd_dq_convert_cl"), stream);
+        bwd_dq_convert_cl<T><<<dim3(unsigned((nq + 63) / 64), unsigned(std::min<int64_t>(a.batch, 65535))), 256, 0, stream>>>(
+            acc, reinterpret_cast<T*>(a.d_q), a.batch, nq, qp, a.heads, p.scale);
         return cudaGetLastError();
       } else {
         const int64_t n8 = a.batch * int64_t(D) * qp / 8;
         const int blocks = int(std::min<int64_t>((n8 + 255) / 256, 148 * 16));
-        ScopedKernel timed("bwd_dq_convert", stream);
-        bwd_dq_convert<<<blocks, 256, 0, stream>>>(reinterpret_cast<const float4*>(acc),
+        ScopedKernel timed((kBf16 ? "bwd_dq_convert_bf16" : "bwd_dq_convert"), stream);
+        bwd_dq_convert<T><<<blocks, 256, 0, stream>>>(reinterpret_cast<const float4*>(acc),
                                                    reinterpret_cast<uint4*>(a.d_q), n8, p.scale);
         return cudaGetLastError();
       }
     }
   }
   if (a.grad_acc) return cudaErrorNotSupported;   // only the fused kernel accumulates (checked by the caller)
-  if (!bwd_maps<D, VD, CL>(&p, a, kBM, kBN)) return cudaErrorInvalidValue;   // dQ kernels: resident queries
+  if (!bwd_maps<T, D, VD, CL>(&p, a, kBM, kBN)) return cudaErrorInvalidValue;   // dQ kernels: resident queries
   bool dq_done = false;
   if constexpr (D == 64 && VD == 64) {
     if (a.variant != 4) {
-      auto kern = split ? bwd_dq_small_kernel<D, VD, true, CL> : bwd_dq_small_kernel<D, VD, false, CL>;
+      auto kern = split ? bwd_dq_small_kernel<T, D, VD, true, CL> : bwd_dq_small_kernel<T, D, VD, false, CL>;
       cudaError_t e =
           plan::ensure_smem(kern, DqSmallCfg<D, VD>::kSmemBytes);
       if (e != cudaSuccess) return e;
       p.n_blocks = (nq + kBM - 1) / kBM;
-      ScopedKernel timed(CL ? "bwd_dq_f16_sm100_2cta_cl" : "bwd_dq_f16_sm100_2cta", stream);
+      ScopedKernel timed(CL ? (kBf16 ? "bwd_dq_bf16_sm100_2cta_cl" : "bwd_dq_f16_sm100_2cta_cl") : (kBf16 ? "bwd_dq_bf16_sm100_2cta" : "bwd_dq_f16_sm100_2cta"), stream);
       kern<<<unsigned(int64_t(p.n_blocks) * p.batch), kBwdThreads, DqSmallCfg<D, VD>::kSmemBytes, stream>>>(p);
       e = cudaGetLastError();
       if (e != cudaSuccess) return e;
@@ -2124,35 +2140,35 @@ cudaError_t launch_bwd(const LaunchArgs& a, cudaStream_t stream) {
     }
   }
   if (!dq_done) {
-    auto kern = split ? bwd_dq_kernel<D, VD, true, CL> : bwd_dq_kernel<D, VD, false, CL>;
+    auto kern = split ? bwd_dq_kernel<T, D, VD, true, CL> : bwd_dq_kernel<T, D, VD, false, CL>;
     cudaError_t e = plan::ensure_smem(kern, DqCfg<D, VD>::kSmemBytes);
     if (e != cudaSuccess) return e;
     p.n_blocks = (nq + 2 * kBM - 1) / (2 * kBM);
-    ScopedKernel timed(CL ? "bwd_dq_f16_sm100_cl" : "bwd_dq_f16_sm100", stream);
+    ScopedKernel timed(CL ? (kBf16 ? "bwd_dq_bf16_sm100_cl" : "bwd_dq_f16_sm100_cl") : (kBf16 ? "bwd_dq_bf16_sm100" : "bwd_dq_f16_sm100"), stream);
     kern<<<unsigned(int64_t(p.n_blocks) * p.batch), kBwdThreads, DqCfg<D, VD>::kSmemBytes, stream>>>(p);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }
-  if (CL && !bwd_maps<D, VD, CL>(&p, a, kBN, kBM)) return cudaErrorInvalidValue;   // dK/dV kernels: resident keys
+  if (CL && !bwd_maps<T, D, VD, CL>(&p, a, kBN, kBM)) return cudaErrorInvalidValue;   // dK/dV kernels: resident keys
   if constexpr (D == 64 && VD == 64) {
     if (a.variant != 4) {
-      auto kern = split ? bwd_dkdv_small_kernel<D, VD, true, CL> : bwd_dkdv_small_kernel<D, VD, false, CL>;
+      auto kern = split ? bwd_dkdv_small_kernel<T, D, VD, true, CL> : bwd_dkdv_small_kernel<T, D, VD, false, CL>;
       cudaError_t e =
           plan::ensure_smem(kern, DkvSmallCfg<D, VD>::kSmemBytes);
       if (e != cudaSuccess) return e;
       p.n_blocks = (nk + kBM - 1) / kBM;
-      ScopedKernel timed(CL ? "bwd_dkdv_f16_sm100_2cta_cl" : "bwd_dkdv_f16_sm100_2cta", stream);
+      ScopedKernel timed(CL ? (kBf16 ? "bwd_dkdv_bf16_sm100_2cta_cl" : "bwd_dkdv_f16_sm100_2cta_cl") : (kBf16 ? "bwd_dkdv_bf16_sm100_2cta" : "bwd_dkdv_f16_sm100_2cta"), stream);
       kern<<<unsigned(int64_t(p.n_blocks) * p.batch), kBwdThreads, DkvSmallCfg<D, VD>::kSmemBytes, stream>>>(p);
       return cudaGetLastError();
     }
   }
   {
-    auto kern = split ? bwd_dkdv_kernel<D, VD, true, CL> : bwd_dkdv_kernel<D, VD, false, CL>;
+    auto kern = split ? bwd_dkdv_kernel<T, D, VD, true, CL> : bwd_dkdv_kernel<T, D, VD, false, CL>;
     cudaError_t e =
         plan::ensure_smem(kern, DkvCfg<D, VD>::kSmemBytes);
     if (e != cudaSuccess) return e;
     p.n_blocks = (nk + kBM - 1) / kBM;
-    ScopedKernel timed(CL ? "bwd_dkdv_f16_sm100_cl" : "bwd_dkdv_f16_sm100", stream);
+    ScopedKernel timed(CL ? (kBf16 ? "bwd_dkdv_bf16_sm100_cl" : "bwd_dkdv_f16_sm100_cl") : (kBf16 ? "bwd_dkdv_bf16_sm100" : "bwd_dkdv_f16_sm100"), stream);
     kern<<<unsigned(int64_t(p.n_blocks) * p.batch), kBwdThreads, DkvCfg<D, VD>::kSmemBytes, stream>>>(p);
     return cudaGetLastError();
   }
@@ -2196,7 +2212,7 @@ BwdLayout bwd_layout(const LaunchArgs& a) {
 static bool aligned16b(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 bool sm100_f16_backward_supports(const LaunchArgs& a) {
-  if (a.dtype != 0) return false;
+  if (a.dtype != 0 && a.dtype != 3) return false;
   if (a.layout == 1) {
     if (a.heads < 1 || a.batch % a.heads) return false;
     if (a.d % 8 || a.v_d % 8) return false;   // strides of the 4-D tensor maps are multiples of 16 bytes
@@ -2232,16 +2248,20 @@ bool sm100_f16_backward_accumulate_supports(const LaunchArgs& a) {
   return true;
 }
 
-template <bool CL>
+template <typename T, bool CL>
 static cudaError_t backward_dispatch_layout(const LaunchArgs& a, cudaStream_t stream) {
   const bool d_small = a.d <= 64, v_small = a.v_d <= 64;
-  if (!d_small && !v_small) return sm100::launch_bwd<128, 128, CL>(a, stream);
-  if (d_small && v_small) return sm100::launch_bwd<64, 64, CL>(a, stream);
-  if (!d_small) return sm100::launch_bwd<128, 64, CL>(a, stream);
-  return sm100::launch_bwd<64, 128, CL>(a, stream);
+  if (!d_small && !v_small) return sm100::launch_bwd<T, 128, 128, CL>(a, stream);
+  if (d_small && v_small) return sm100::launch_bwd<T, 64, 64, CL>(a, stream);
+  if (!d_small) return sm100::launch_bwd<T, 128, 64, CL>(a, stream);
+  return sm100::launch_bwd<T, 64, 128, CL>(a, stream);
+}
+template <typename T>
+static cudaError_t backward_dispatch_t(const LaunchArgs& a, cudaStream_t stream) {
+  return a.layout == 1 ? backward_dispatch_layout<T, true>(a, stream) : backward_dispatch_layout<T, false>(a, stream);
 }
 static cudaError_t backward_dispatch(const LaunchArgs& a, cudaStream_t stream) {
-  return a.layout == 1 ? backward_dispatch_layout<true>(a, stream) : backward_dispatch_layout<false>(a, stream);
+  return a.dtype == 3 ? backward_dispatch_t<__nv_bfloat16>(a, stream) : backward_dispatch_t<__half>(a, stream);
 }
 
 cudaError_t sm100_f16_backward(const LaunchArgs& a0, cudaStream_t stream) {

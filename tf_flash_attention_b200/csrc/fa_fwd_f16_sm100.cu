@@ -1,4 +1,4 @@
-// fa_fwd_f16_sm100.cu — Blackwell-native fp16 forward: TMA -> swizzled smem -> tcgen05.mma with
+// fa_fwd_f16_sm100.cu — Blackwell-native 16-bit (fp16 / bf16) forward: TMA -> swizzled smem -> tcgen05.mma with
 // TMEM accumulators, warp-specialised (1 TMA producer warp, 1 MMA issuer warp, 2 softmax
 // warpgroups that ping-pong over two 128-row Q tiles).
 //
@@ -10,7 +10,7 @@
 // Layout facts this design leans on (channel-first tensors, sequence contiguous):
 //   S = Q K^T : A = Q tile, B = K tile, both "MN-major" in shared memory (the 64-element swizzle
 //               row runs along the sequence, 8 channels form one 1024-byte swizzle atom)
-//   O = P V   : A = P (fp16, written by the softmax warps into TMEM over S), B = V tile, K-major
+//   O = P V   : A = P (fp16 / bf16, written by the softmax warps into TMEM over S), B = V tile, K-major
 // so no transposes are needed anywhere.
 #include "fa_common.cuh"
 #include "fa_launch.h"
@@ -19,6 +19,8 @@
 #include "sm100_tiles.cuh"
 
 #include <cudaTypedefs.h>
+
+#include <type_traits>
 
 namespace fa {
 namespace sm100 {
@@ -37,7 +39,7 @@ struct alignas(64) FwdParams {
   CUtensorMap map_q, map_k, map_v, map_o;
   FaRule rule;
   float* l;
-  __half* m;
+  void* m;         // T [batch][nq]
   int32_t nq, nk, n_qpairs;
   int32_t batch;
   int32_t heads;   // channel-last tensors: batch element = outer * heads + head
@@ -89,7 +91,8 @@ struct FwdCfg {
 // positions of one head): the same tiles with positions and channels swapped, so every shared-memory operand flips
 // between MN-major and K-major (sm100_ptx.cuh tile_desc) and O is staged row-major. Products, accumulation order and
 // results are identical to the channel-first kernel's.
-template <int D, int VD, int BN, int MINB, bool CL>
+// T = __half or __nv_bfloat16: the element type of Q, K, V, O, m and of P in tensor memory.
+template <typename T, int D, int VD, int BN, int MINB, bool CL>
 __global__ void __launch_bounds__(kThreads, MINB) fwd_kernel(const __grid_constant__ FwdParams p) {
   using Cfg = FwdCfg<D, VD, BN>;
   constexpr int kBlockN = BN;
@@ -224,8 +227,8 @@ __global__ void __launch_bounds__(kThreads, MINB) fwd_kernel(const __grid_consta
         TileIter it;
         it.init(sched, 2, kt_first, kt_last);
         const int n = it.count();
-        constexpr uint32_t idesc_qk = idesc_f16(kBlockM, kBlockN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
-        constexpr uint32_t idesc_pv = idesc_f16(kBlockM, VD, false, tile_mn_major<CL>(false));
+        constexpr uint32_t idesc_qk = idesc_16<T>(kBlockM, kBlockN, tile_mn_major<CL>(true), tile_mn_major<CL>(true));
+        constexpr uint32_t idesc_pv = idesc_16<T>(kBlockM, VD, false, tile_mn_major<CL>(false));
         auto issue_qk = [&](int i, int stage) {
           const uint32_t a0 = q_smem + i * Cfg::kQTileBytes;
           const uint32_t b0 = kv_smem + stage * Cfg::kStageBytes;
@@ -402,17 +405,17 @@ __global__ void __launch_bounds__(kThreads, MINB) fwd_kernel(const __grid_consta
       }
       const float m_use = (m_ref == NEG_INF) ? 0.f : m_ref;
       float sum0 = 0.f, sum1 = 0.f;
-      auto exp_cols = [&](int c0, int n, uint32_t* pk) {   // columns [c0, c0 + n) -> fp16 pairs
+      auto exp_cols = [&](int c0, int n, uint32_t* pk) {   // columns [c0, c0 + n) -> pairs of T
 #pragma unroll
         for (int e = 0; e < n; e += 2) {
           const float p0 = ex2(fmaf(s[c0 + e], scale_log2, -m_use));
           const float p1 = ex2(fmaf(s[c0 + e + 1], scale_log2, -m_use));
           sum0 += p0;
           sum1 += p1;
-          pk[e >> 1] = pack_half2(p0, p1);
+          pk[e >> 1] = pack2<T>(p0, p1);
         }
       };
-      // P = exp2(S*scale*log2e - m) -> fp16 pairs written over S, 32 columns at a time
+      // P = exp2(S*scale*log2e - m) -> pairs of T written over S, 32 columns at a time
       if constexpr (Cfg::kHalves) {
         exp_cols(0, 32, pk0);
         tmem_st16(t_s + 0, pk0);
@@ -441,9 +444,9 @@ __global__ void __launch_bounds__(kThreads, MINB) fwd_kernel(const __grid_consta
       ++j;
     }
 
-    // ---- epilogue: O = acc / l -> fp16 -> smem [VD][64] x2 -> TMA store; l, m -> global ----
+    // ---- epilogue: O = acc / l -> T -> smem [VD][64] x2 -> TMA store; l, m -> global ----
     uint8_t* stage_gen = smem_gen + i * Cfg::kQTileBytes;
-    __half* stage_h = reinterpret_cast<__half*>(stage_gen) + (r >> 6) * (VD * 64) + (r & 63);
+    T* stage_h = reinterpret_cast<T*>(stage_gen) + (r >> 6) * (VD * 64) + (r & 63);
     if (j > 0) {
       mbar_wait(bar_o_final + 8 * i, 0);
       tc_fence_after();
@@ -457,15 +460,15 @@ __global__ void __launch_bounds__(kThreads, MINB) fwd_kernel(const __grid_consta
 #pragma unroll
           for (int e = 0; e < 32; e += 8) {
             uint4 w;
-            w.x = pack_half2(o[e] * inv, o[e + 1] * inv);       // inv = 0 for rows without keys
-            w.y = pack_half2(o[e + 2] * inv, o[e + 3] * inv);
-            w.z = pack_half2(o[e + 4] * inv, o[e + 5] * inv);
-            w.w = pack_half2(o[e + 6] * inv, o[e + 7] * inv);
+            w.x = pack2<T>(o[e] * inv, o[e + 1] * inv);       // inv = 0 for rows without keys
+            w.y = pack2<T>(o[e + 2] * inv, o[e + 3] * inv);
+            w.z = pack2<T>(o[e + 4] * inv, o[e + 5] * inv);
+            w.w = pack2<T>(o[e + 6] * inv, o[e + 7] * inv);
             *reinterpret_cast<uint4*>(stage_gen + cl_chunk_offset(r, c * 32 + e, kBlockM)) = w;
           }
         } else {
 #pragma unroll
-          for (int e = 0; e < 32; ++e) stage_h[(c * 32 + e) * 64] = __float2half_rn(l_sum > 0.f ? o[e] * inv : 0.f);
+          for (int e = 0; e < 32; ++e) stage_h[(c * 32 + e) * 64] = from_acc<T>(l_sum > 0.f ? o[e] * inv : 0.f);
         }
       }
     } else {
@@ -477,17 +480,18 @@ __global__ void __launch_bounds__(kThreads, MINB) fwd_kernel(const __grid_consta
           *reinterpret_cast<uint4*>(stage_gen + cl_chunk_offset(r, c, kBlockM)) = make_uint4(0, 0, 0, 0);
       } else {
 #pragma unroll 8
-        for (int c = 0; c < VD; ++c) stage_h[c * 64] = __float2half_rn(0.f);
+        for (int c = 0; c < VD; ++c) stage_h[c * 64] = from_acc<T>(0.f);
       }
     }
     if (q_valid) {
       const int64_t idx = int64_t(b) * p.nq + qi;
+      T* m = static_cast<T*>(p.m);
       if (l_sum > 0.f) {
-        const __half m_h = __float2half_rn(m_true * kLn2);
-        p.m[idx] = m_h;
-        p.l[idx] = l_sum * ex2(m_ref - __half2float(m_h) * kLog2e);
+        const T m_h = from_acc<T>(m_true * kLn2);
+        m[idx] = m_h;
+        p.l[idx] = l_sum * ex2(m_ref - to_acc<float>(m_h) * kLog2e);
       } else {
-        p.m[idx] = sentinel<__half>();
+        m[idx] = sentinel<T>();
         p.l[idx] = 0.f;
       }
     }
@@ -527,65 +531,70 @@ bool make_map_2d(CUtensorMap* map, const void* base, int64_t rows, int64_t cols,
                           swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
-// 3-D view [batch][channels][sequence] of a channel-first fp16 tensor (`pitch` elements between channel rows): the box is
-// 64 positions x box_rows channels of one batch element; channels past `channels` are zero-filled / clipped.
+// 3-D view [batch][channels][sequence] of a channel-first 16-bit tensor (`pitch` elements between channel rows): the box
+// is 64 positions x box_rows channels of one batch element; channels past `channels` are zero-filled / clipped.
 bool make_map_3d(CUtensorMap* map, const void* base, int64_t batch, int64_t channels, int64_t seq, int64_t pitch,
-                 int box_rows, bool swizzle128) {
+                 int box_rows, bool swizzle128, CUtensorMapDataType dtype) {
   const uint64_t gdim[3] = {uint64_t(seq), uint64_t(channels), uint64_t(batch)};
   const uint64_t gstride[2] = {uint64_t(pitch) * 2, uint64_t(pitch) * 2 * uint64_t(channels)};
   const uint32_t box[3] = {64u, uint32_t(box_rows), 1u};
-  return plan::tensor_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, base, gdim, gstride, box,
+  return plan::tensor_map(map, dtype, 3, base, gdim, gstride, box,
                           swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
-// 4-D view [outer][sequence][heads][channels] of a channel-last fp16 tensor: the box is 64 channels x box_rows positions
+// 4-D view [outer][sequence][heads][channels] of a channel-last 16-bit tensor: the box is 64 channels x box_rows positions
 // of one head (one 128-byte-row slab of a tile); channels past `channels` and positions past `seq` are zero-filled on
 // loads and clipped on stores.
 bool make_map_cl(CUtensorMap* map, const void* base, int64_t outer, int64_t heads, int64_t channels, int64_t seq,
-                 int box_rows) {
+                 int box_rows, CUtensorMapDataType dtype) {
   const uint64_t gdim[4] = {uint64_t(channels), uint64_t(heads), uint64_t(seq), uint64_t(outer)};
   const uint64_t gstride[3] = {uint64_t(channels) * 2, uint64_t(channels) * 2 * uint64_t(heads),
                                uint64_t(channels) * 2 * uint64_t(heads) * uint64_t(seq)};
   const uint32_t box[4] = {64u, 1u, uint32_t(box_rows), 1u};
-  return plan::tensor_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, base, gdim, gstride, box, CU_TENSOR_MAP_SWIZZLE_128B);
+  return plan::tensor_map(map, dtype, 4, base, gdim, gstride, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-template <int D, int VD, int BN, int MINB, bool CL>
+template <typename T, int D, int VD, int BN, int MINB, bool CL>
 cudaError_t launch_fwd(const LaunchArgs& a, cudaStream_t stream) {
   using Cfg = FwdCfg<D, VD, BN>;
+  constexpr CUtensorMapDataType dt = Elt16<T>::kTmaType;
+  constexpr bool bf16 = std::is_same<T, __nv_bfloat16>::value;
   FwdParams p;
   const int nq = a.rule.q.total, nk = a.rule.k.total;
   // D, VD are the kernel's padded channel counts (a.d <= D, a.v_d <= VD)
   if constexpr (CL) {
     const int64_t heads = a.heads > 0 ? a.heads : 1, outer = a.batch / heads;
-    if (!make_map_cl(&p.map_q, a.q, outer, heads, a.d, nq, kBlockM) ||
-        !make_map_cl(&p.map_k, a.k, outer, heads, a.d, nk, BN) ||
-        !make_map_cl(&p.map_v, a.v, outer, heads, a.v_d, nk, BN) ||
-        !make_map_cl(&p.map_o, a.o, outer, heads, a.v_d, nq, kBlockM))
+    if (!make_map_cl(&p.map_q, a.q, outer, heads, a.d, nq, kBlockM, dt) ||
+        !make_map_cl(&p.map_k, a.k, outer, heads, a.d, nk, BN, dt) ||
+        !make_map_cl(&p.map_v, a.v, outer, heads, a.v_d, nk, BN, dt) ||
+        !make_map_cl(&p.map_o, a.o, outer, heads, a.v_d, nq, kBlockM, dt))
       return cudaErrorInvalidValue;
     p.heads = int32_t(heads);
   } else {
     const int64_t qp = a.q_pitch ? a.q_pitch : nq, kp = a.k_pitch ? a.k_pitch : nk;
-    if (!make_map_3d(&p.map_q, a.q, a.batch, a.d, nq, qp, D, true) ||
-        !make_map_3d(&p.map_k, a.k, a.batch, a.d, nk, kp, D, true) ||
-        !make_map_3d(&p.map_v, a.v, a.batch, a.v_d, nk, kp, VD, true) ||
-        !make_map_3d(&p.map_o, a.o, a.batch, a.v_d, nq, qp, VD, false))
+    if (!make_map_3d(&p.map_q, a.q, a.batch, a.d, nq, qp, D, true, dt) ||
+        !make_map_3d(&p.map_k, a.k, a.batch, a.d, nk, kp, D, true, dt) ||
+        !make_map_3d(&p.map_v, a.v, a.batch, a.v_d, nk, kp, VD, true, dt) ||
+        !make_map_3d(&p.map_o, a.o, a.batch, a.v_d, nq, qp, VD, false, dt))
       return cudaErrorInvalidValue;
     p.heads = 1;
   }
   p.rule = a.rule;
   p.l = (float*)a.l;
-  p.m = (__half*)a.m;
+  p.m = a.m;
   p.nq = nq;
   p.nk = nk;
   p.n_qpairs = (nq + kQTiles * kBlockM - 1) / (kQTiles * kBlockM);
   p.batch = int32_t(a.batch);
   p.scale_log2 = kLog2e / sqrtf(float(a.d));
-  auto kern = fwd_kernel<D, VD, BN, MINB, CL>;
+  auto kern = fwd_kernel<T, D, VD, BN, MINB, CL>;
   cudaError_t e = plan::ensure_smem(kern, Cfg::kSmemBytes);
   if (e != cudaSuccess) return e;
-  ScopedKernel timed(CL ? (BN == 128 ? "fwd_f16_sm100_cl" : "fwd_f16_sm100_n64_cl")
-                        : (BN == 128 ? "fwd_f16_sm100" : "fwd_f16_sm100_n64"), stream);
+  const char* name = bf16 ? (CL ? (BN == 128 ? "fwd_bf16_sm100_cl" : "fwd_bf16_sm100_n64_cl")
+                                 : (BN == 128 ? "fwd_bf16_sm100" : "fwd_bf16_sm100_n64"))
+                          : (CL ? (BN == 128 ? "fwd_f16_sm100_cl" : "fwd_f16_sm100_n64_cl")
+                                : (BN == 128 ? "fwd_f16_sm100" : "fwd_f16_sm100_n64"));
+  ScopedKernel timed(name, stream);
   kern<<<unsigned(int64_t(p.n_qpairs) * p.batch), kThreads, Cfg::kSmemBytes, stream>>>(p);
   return cudaGetLastError();
 }
@@ -628,7 +637,7 @@ static FwdPack fwd_pack_layout(const LaunchArgs& a) {
 // lengths (packed to a 16-byte pitch when needed): the shapes the reference's own tests draw (tests/test_1d.py:57-66,
 // test_2d.py:85-94: channels 8..32, arbitrary even lengths) run on the tensor cores.
 bool sm100_f16_forward_supports(const LaunchArgs& a) {
-  if (a.dtype != 0 || a.accumulate) return false;
+  if ((a.dtype != 0 && a.dtype != 3) || a.accumulate) return false;
   if (a.d < 1 || a.v_d < 1 || a.d > 128 || a.v_d > 128) return false;
   const int64_t nq = a.rule.q.total, nk = a.rule.k.total;
   const FwdPack w = fwd_pack_layout(a);
@@ -663,19 +672,23 @@ size_t sm100_f16_workspace_bytes(const LaunchArgs& a, bool backward) {
 // head_dim <= 64: the 64-key / two-CTAs-per-SM configuration is faster on every workload measured (S1 1.01 -> 0.67 ms,
 // S2 3.95 -> 2.01 ms, C3 0.84 -> 0.51 ms, C4 0.86 -> 0.73 ms; profiles/r1_short_sequences.md); override 5 keeps the
 // 128-key / one-CTA configuration reachable for A/B runs.
-template <bool CL>
+template <typename T, bool CL>
 static cudaError_t forward_dispatch_layout(const LaunchArgs& a, cudaStream_t stream) {
   const bool d_small = a.d <= 64, v_small = a.v_d <= 64;
-  if (!d_small && !v_small) return sm100::launch_fwd<128, 128, 128, 1, CL>(a, stream);
+  if (!d_small && !v_small) return sm100::launch_fwd<T, 128, 128, 128, 1, CL>(a, stream);
   if (d_small && v_small) {
-    if (a.variant != 5) return sm100::launch_fwd<64, 64, 64, 2, CL>(a, stream);
-    return sm100::launch_fwd<64, 64, 128, 1, CL>(a, stream);
+    if (a.variant != 5) return sm100::launch_fwd<T, 64, 64, 64, 2, CL>(a, stream);
+    return sm100::launch_fwd<T, 64, 64, 128, 1, CL>(a, stream);
   }
-  if (!d_small) return sm100::launch_fwd<128, 64, 128, 1, CL>(a, stream);
-  return sm100::launch_fwd<64, 128, 128, 1, CL>(a, stream);
+  if (!d_small) return sm100::launch_fwd<T, 128, 64, 128, 1, CL>(a, stream);
+  return sm100::launch_fwd<T, 64, 128, 128, 1, CL>(a, stream);
+}
+template <typename T>
+static cudaError_t forward_dispatch_t(const LaunchArgs& a, cudaStream_t stream) {
+  return a.layout == 1 ? forward_dispatch_layout<T, true>(a, stream) : forward_dispatch_layout<T, false>(a, stream);
 }
 static cudaError_t forward_dispatch(const LaunchArgs& a, cudaStream_t stream) {
-  return a.layout == 1 ? forward_dispatch_layout<true>(a, stream) : forward_dispatch_layout<false>(a, stream);
+  return a.dtype == 3 ? forward_dispatch_t<__nv_bfloat16>(a, stream) : forward_dispatch_t<__half>(a, stream);
 }
 
 cudaError_t sm100_f16_forward(const LaunchArgs& a0, cudaStream_t stream) {

@@ -844,6 +844,7 @@ bool generic_supports(const LaunchArgs& a, bool backward) {
   if (a.d <= 256 && a.v_d <= 256) return true;
   switch (a.dtype) {
     case 0: return generic::wide_grid_fits<__half>(a, backward);
+    case 3: return generic::wide_grid_fits<__nv_bfloat16>(a, backward);
     case 1: return generic::wide_grid_fits<float>(a, backward);
     default: return generic::wide_grid_fits<double>(a, backward);
   }
@@ -857,6 +858,7 @@ size_t generic_workspace_bytes(int dtype, int64_t batch, int64_t nq, bool backwa
 cudaError_t generic_forward(const LaunchArgs& a, cudaStream_t stream) {
   switch (a.dtype) {
     case 0: return generic::forward_t<__half>(a, stream);
+    case 3: return generic::forward_t<__nv_bfloat16>(a, stream);
     case 1: return generic::forward_t<float>(a, stream);
     default: return generic::forward_t<double>(a, stream);
   }
@@ -865,6 +867,7 @@ cudaError_t generic_forward(const LaunchArgs& a, cudaStream_t stream) {
 cudaError_t generic_backward(const LaunchArgs& a, cudaStream_t stream) {
   switch (a.dtype) {
     case 0: return generic::backward_t<__half>(a, stream);
+    case 3: return generic::backward_t<__nv_bfloat16>(a, stream);
     case 1: return generic::backward_t<float>(a, stream);
     default: return generic::backward_t<double>(a, stream);
   }

@@ -209,7 +209,9 @@ static cudaError_t layout_t(const void* x, void* y, int64_t B, int64_t S, int32_
 cudaError_t layout_transpose(int dtype, const void* x, void* y, int64_t B, int64_t S, int32_t H, int32_t C,
                              int to_channel_first, int variant, cudaStream_t stream) {
   switch (dtype) {
-    case 0: return layout_t<__half>(x, y, B, S, H, C, to_channel_first, variant, stream);
+    case 0:
+    case 3:   // bf16 moves the same 2-byte words: the fp16 kernels on reinterpreted pointers, bit-exact
+      return layout_t<__half>(x, y, B, S, H, C, to_channel_first, variant, stream);
     case 1: return layout_t<float>(x, y, B, S, H, C, to_channel_first, variant, stream);
     default: return layout_t<double>(x, y, B, S, H, C, to_channel_first, variant, stream);
   }

@@ -227,8 +227,8 @@ int fa_ring_destroy(fa_ring_t* r) {
 namespace {
 
 size_t al256(size_t n) { return (n + 255) & ~size_t(255); }
-size_t elt(int dtype) { return dtype == FA_F16 ? 2 : dtype == FA_F32 ? 4 : 8; }
-size_t l_elt(int dtype) { return dtype == FA_F64 ? 8 : 4; }     // l is float for half
+size_t elt(int dtype) { return dtype == FA_F16 || dtype == FA_BF16 ? 2 : dtype == FA_F32 ? 4 : 8; }
+size_t l_elt(int dtype) { return dtype == FA_F64 ? 8 : 4; }     // l is float for half and bf16
 size_t acc_elt(int dtype) { return dtype == FA_F64 ? 8 : 4; }   // accumulators: float (double for f64)
 
 fa_problem_t chunk_problem(int dtype, int rule, int64_t batch, int d, int v_d, int c, int64_t full_len) {
@@ -307,7 +307,7 @@ RingArena ring_arena(int dtype, int64_t batch, int d, int v_d, int c, int world,
   } while (0)
 
 int ring_args_ok(fa_ring_t* kv, int dtype, int64_t batch, int d, int v_d, int c) {
-  if (dtype < FA_F16 || dtype > FA_F64) return FA_EINVAL_DTYPE;
+  if (dtype < FA_F16 || dtype > FA_BF16) return FA_EINVAL_DTYPE;
   if (batch < 1 || d < 1 || v_d < 1 || c < 1) return FA_EINVAL_SHAPE;
   if (kv && (kv->world < 1 || kv->n_slots < 2)) return FA_EINVAL_SHAPE;
   return FA_OK;
@@ -319,12 +319,12 @@ extern "C" {
 
 size_t fa_ring_causal_arena_bytes(int32_t dtype, int64_t batch, int32_t d, int32_t v_d, int32_t chunk, int32_t world,
                                   int32_t backward) {
-  if (dtype < FA_F16 || dtype > FA_F64 || batch < 1 || d < 1 || v_d < 1 || chunk < 1 || world < 1) return 0;
+  if (dtype < FA_F16 || dtype > FA_BF16 || batch < 1 || d < 1 || v_d < 1 || chunk < 1 || world < 1) return 0;
   return ring_arena(dtype, batch, d, v_d, chunk, world, backward != 0).total;
 }
 
 size_t fa_ring_causal_slot_bytes(int32_t dtype, int64_t batch, int32_t d, int32_t v_d, int32_t chunk, int32_t accumulators) {
-  if (dtype < FA_F16 || dtype > FA_F64 || batch < 1 || d < 1 || v_d < 1 || chunk < 1) return 0;
+  if (dtype < FA_F16 || dtype > FA_BF16 || batch < 1 || d < 1 || v_d < 1 || chunk < 1) return 0;
   const size_t e = accumulators ? acc_elt(dtype) : elt(dtype);
   return al256(size_t(2) * batch * d * chunk * e) + al256(size_t(2) * batch * v_d * chunk * e);
 }

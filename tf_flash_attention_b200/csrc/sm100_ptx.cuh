@@ -3,8 +3,11 @@
 // ld / st / fences), setmaxnreg, named barriers. Hand-written; no CuTe / CUTLASS.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <stdint.h>
+
+#include "fa_common.cuh"
 
 namespace fa {
 namespace ptx {
@@ -285,6 +288,23 @@ __host__ __device__ constexpr uint32_t idesc_f16(int m, int n, bool a_mn_major, 
          (uint32_t(m >> 4) << 24);
 }
 
+// 16-bit element types of the tcgen05 kernels: fp16 and bf16 share every tile, descriptor and schedule; they differ in
+// the a/b format bits of the kind::f16 instruction descriptor (0 = F16, 1 = BF16), the TMA data type and the float
+// conversions.
+template <typename T> struct Elt16;
+template <> struct Elt16<__half> {
+  static constexpr uint32_t kFormat = 0;
+  static constexpr CUtensorMapDataType kTmaType = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+};
+template <> struct Elt16<__nv_bfloat16> {
+  static constexpr uint32_t kFormat = 1;
+  static constexpr CUtensorMapDataType kTmaType = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+};
+template <typename T>
+__host__ __device__ constexpr uint32_t idesc_16(int m, int n, bool a_mn_major, bool b_mn_major) {
+  return idesc_f16(m, n, a_mn_major, b_mn_major) | (Elt16<T>::kFormat << 7) | (Elt16<T>::kFormat << 10);
+}
+
 // Instruction descriptor for kind::tf32 (a/b format 2 = TF32) with F32 accumulation.
 __host__ __device__ constexpr uint32_t idesc_tf32(int m, int n, bool a_mn_major, bool b_mn_major) {
   return (1u << 4) | (2u << 7) | (2u << 10) | (uint32_t(a_mn_major) << 15) | (uint32_t(b_mn_major) << 16) |
@@ -312,6 +332,14 @@ __device__ __forceinline__ float ex2(float x) {
 __device__ __forceinline__ uint32_t pack_half2(float lo, float hi) {
   __half2 h = __floats2half2_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&h);
+}
+// two floats -> one 32-bit word of two T (round to nearest even; `lo` in the low half)
+template <typename T> __device__ __forceinline__ uint32_t pack2(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t pack2<__half>(float lo, float hi) { return pack_half2(lo, hi); }
+template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float lo, float hi) {
+  uint32_t r;   // cvt packs its first source into the upper half
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
 }
 
 
@@ -349,27 +377,28 @@ __device__ __forceinline__ void tile_store(const void* map, uint32_t src, int po
       if (pos0 + h * 64 < n) tma_store_bc(map, src + h * (C * 128), pos0 + h * 64, bc.b);
   }
 }
-// One thread owns row r of an output tile and stages channels [c0, c0 + 32) = v[0..32) * scale as fp16.
+// One thread owns row r of an output tile and stages channels [c0, c0 + 32) = v[0..32) * scale as T.
 // channel-first: [C][64] per 64 positions, unswizzled (lanes = consecutive positions: conflict-free 2-byte stores);
 // channel-last: slabs of 64 channels, rows of 128 bytes with TMA's 128-byte swizzle (16-byte stores, conflict-free)
-template <bool CL>
+template <bool CL, typename T>
 __device__ __forceinline__ void stage_row32(uint8_t* tile, int r, int c0, int R, int C, const float* v, float scale) {
   if constexpr (CL) {
 #pragma unroll
     for (int e = 0; e < 32; e += 8) {
       uint4 w;
-      w.x = pack_half2(v[e] * scale, v[e + 1] * scale);
-      w.y = pack_half2(v[e + 2] * scale, v[e + 3] * scale);
-      w.z = pack_half2(v[e + 4] * scale, v[e + 5] * scale);
-      w.w = pack_half2(v[e + 6] * scale, v[e + 7] * scale);
+      w.x = pack2<T>(v[e] * scale, v[e + 1] * scale);
+      w.y = pack2<T>(v[e + 2] * scale, v[e + 3] * scale);
+      w.z = pack2<T>(v[e + 4] * scale, v[e + 5] * scale);
+      w.w = pack2<T>(v[e + 6] * scale, v[e + 7] * scale);
       *reinterpret_cast<uint4*>(tile + cl_chunk_offset(r, c0 + e, R)) = w;
     }
   } else {
-    __half* h = reinterpret_cast<__half*>(tile) + (r >> 6) * (C * 64) + (r & 63);
+    T* h = reinterpret_cast<T*>(tile) + (r >> 6) * (C * 64) + (r & 63);
 #pragma unroll
-    for (int e = 0; e < 32; ++e) h[(c0 + e) * 64] = __float2half_rn(v[e] * scale);
+    for (int e = 0; e < 32; ++e) h[(c0 + e) * 64] = from_acc<T>(v[e] * scale);
   }
 }
+// zeros are the same bits in fp16 and bf16: one version serves both
 template <bool CL>
 __device__ __forceinline__ void stage_row_zero(uint8_t* tile, int r, int c_begin, int c_end, int R, int C) {
   if constexpr (CL) {

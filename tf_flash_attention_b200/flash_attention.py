@@ -9,7 +9,8 @@ the same six entry points, argument names, defaults and return convention
   full_2d / causal_2d / local_2d                                          reference :219,266,312
 
 with the same channel-first layouts ``batch_shape + (channel, sequence...)``, the same
-dtypes (float16 / float32 / float64; ``l`` is float32 for float16 inputs) and the
+dtypes (float16 / float32 / float64; ``l`` is float32 for float16 inputs) plus bfloat16 for
+torch tensors (``l`` float32, as for float16; NumPy has no bfloat16), and the
 registered gradient (only ``dO`` is propagated; gradients of ``l`` and ``m`` are
 ignored, reference :374-390).
 
@@ -39,7 +40,13 @@ _NP_L_DTYPE = {_capi.FA_F16: np.float32, _capi.FA_F32: np.float32, _capi.FA_F64:
 
 
 def _torch_codes():
-    return {torch.float16: _capi.FA_F16, torch.float32: _capi.FA_F32, torch.float64: _capi.FA_F64}
+    return {torch.float16: _capi.FA_F16, torch.float32: _capi.FA_F32, torch.float64: _capi.FA_F64,
+            torch.bfloat16: _capi.FA_BF16}
+
+
+def _l_dtype(dtype):
+    """dtype of ``l`` for inputs of `dtype`: float32 for the 16-bit types"""
+    return torch.float32 if dtype in (torch.float16, torch.bfloat16) else dtype
 
 
 def _is_torch(x):
@@ -143,7 +150,7 @@ def _forward_device(p, Q, K, V, out=None):
         raise _capi.FlashAttentionError(-101, "torch inputs must live on a CUDA device (no CPU fallback)")
     Q, K, V = Q.contiguous(), K.contiguous(), V.contiguous()
     o_shape, lm_shape = _out_shapes(p, Q, V)
-    l_dtype = torch.float32 if Q.dtype == torch.float16 else Q.dtype
+    l_dtype = _l_dtype(Q.dtype)
     if out is None:
         O = torch.empty(o_shape, dtype=Q.dtype, device=Q.device)
         l = torch.empty(lm_shape, dtype=l_dtype, device=Q.device)
@@ -268,8 +275,8 @@ def _attend(p, Q, K, V, returning_l_m):
 # public API — same names, argument order and defaults as the reference
 # ------------------------------------------------------------------------------------ #
 # `layout` (keyword only, not in the reference): 'channel_last' takes Q, K, V as outer + sequence + (heads, channels) -
-# what a projection produces - and returns O the same way (l, m: outer + (heads,) + sequence). The fp16 tensor-core
-# kernels read and write that layout directly through their TMA descriptors (SURVEY.md section 8 f3); other dtypes /
+# what a projection produces - and returns O the same way (l, m: outer + (heads,) + sequence). The fp16 / bf16
+# tensor-core kernels read and write that layout directly through their TMA descriptors (SURVEY.md section 8 f3); other dtypes /
 # shapes go through the adapter kernel either side of the channel-first op.
 def full_1d(Q, K, V, sync_mode='none_front', returning_l_m=False, *, layout='channel_first'):
     '''Full attention (no masking) on 1d sequences. Reference: flash_attention.py:80-119.'''
@@ -386,7 +393,7 @@ def _layout(x, to_channel_first):
         raise _capi.InvalidArgumentError(_capi.FA_EINVAL_NULL, "layout adapters take torch CUDA tensors (no CPU fallback)")
     if x.dim() != 4:
         raise _capi.InvalidArgumentError(_capi.FA_EINVAL_RANK, "expected a rank-4 tensor")
-    codes = {torch.float16: _capi.FA_F16, torch.float32: _capi.FA_F32, torch.float64: _capi.FA_F64}
+    codes = _torch_codes()
     if x.dtype not in codes:
         raise _capi.InvalidArgumentError(_capi.FA_EINVAL_DTYPE, f"unsupported dtype {x.dtype}")
     x = x.contiguous()

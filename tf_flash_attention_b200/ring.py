@@ -132,7 +132,7 @@ class DeviceBackend:
     def new_out_like(self, q, v):
         """(O, l, m) buffers for queries q [..., d, c] and values v [..., v_d, c]."""
         t = self.torch
-        ldt = t.float32 if q.dtype == t.float16 else q.dtype
+        ldt = t.float32 if q.dtype in (t.float16, t.bfloat16) else q.dtype
         lead = tuple(q.shape[:-2])
         return (t.empty(lead + (v.shape[-2], q.shape[-1]), dtype=q.dtype, device=q.device),
                 t.empty(lead + (q.shape[-1],), dtype=ldt, device=q.device),
@@ -186,7 +186,7 @@ class DeviceBackend:
 
     def new_out(self, like_q):
         t, dev = self.torch, like_q.device
-        ldt = t.float32 if like_q.dtype == t.float16 else like_q.dtype
+        ldt = t.float32 if like_q.dtype in (t.float16, t.bfloat16) else like_q.dtype
         return (t.empty(self.batch_shape + (self.v_d, self.chunk), dtype=like_q.dtype, device=dev),
                 t.empty(self.batch_shape + (self.chunk,), dtype=ldt, device=dev),
                 t.empty(self.batch_shape + (self.chunk,), dtype=like_q.dtype, device=dev))
@@ -676,7 +676,8 @@ def _causal_ring_setup(Q, V, sync_mode, group):
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     layout = ZigZag(Q.shape[-1] * world, world)
-    codes = {torch.float16: _capi.FA_F16, torch.float32: _capi.FA_F32, torch.float64: _capi.FA_F64}
+    codes = {torch.float16: _capi.FA_F16, torch.float32: _capi.FA_F32, torch.float64: _capi.FA_F64,
+             torch.bfloat16: _capi.FA_BF16}
     backend = DeviceBackend(codes[Q.dtype], "causal", "none_front", 1, 0, False, Q.shape[:-2], Q.shape[-2], V.shape[-2],
                             layout.chunk, layout.seq_len)
     return dist if world > 1 else None, rank, layout, backend
