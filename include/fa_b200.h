@@ -61,7 +61,8 @@ enum {
   FA_EINVAL_STRIDE = -7,       /* log2_stride_size < 0, >= 31 or window<<stride overflows   */
                                /*                                flash_attention.h:90       */
   FA_EINVAL_SHAPE = -8,        /* a dimension < 1, or q/k/orders do not fit int32           */
-  FA_EINVAL_WORKSPACE = -9,    /* workspace smaller than fa_workspace_bytes()               */
+  FA_EINVAL_WORKSPACE = -9,    /* workspace smaller than fa_workspace_bytes(), or needed and */
+                               /* NULL or not 256-byte aligned (host arenas: always)        */
   FA_EINVAL_RANK = -10,        /* fa_check_*_shapes: rank mismatch / rank < seq_dims+2      */
   FA_EINVAL_CHANNEL = -11,     /* fa_check_*_shapes: channel mismatch                       */
   FA_EINVAL_BATCH = -12,       /* fa_check_*_shapes: batch shapes differ                    */
@@ -120,7 +121,8 @@ int fa_backward(const fa_problem_t* p, const void* q, const void* k, const void*
 
 /* Device scratch the caller must provide (replaces the reference's allocate_temp of
  * Br_occupancy, flash_attention_forward.cc:330 / flash_attention_backward.cc:283).
- * May be 0. */
+ * May be 0. When it is not, the workspace must be 256-byte aligned: fa_forward, fa_backward
+ * and fa_backward_accumulate return FA_EINVAL_WORKSPACE before any launch otherwise. */
 size_t fa_workspace_bytes(const fa_problem_t* p, int is_backward);
 
 /* Replaces FlashAttentionLauncher::EstimateForwardFlops (flash_attention.h:254-260,
@@ -207,8 +209,9 @@ int fa_check_backward_shapes(int32_t seq_dims, int32_t rank_q, const int64_t* q_
 
 /* Same contract as fa_forward / fa_backward but every tensor pointer is HOST memory
  * (pinned or pageable). The library stages through the caller-provided device arena
- * `dev_arena` (>= fa_host_arena_bytes), copies in, runs, copies the results back and
- * returns after the stream has drained. Used for the end-to-end number in bench.py. */
+ * `dev_arena` (>= fa_host_arena_bytes, 256-byte aligned, else FA_EINVAL_WORKSPACE), copies
+ * in, runs, copies the results back and returns after the stream has drained. Used for the
+ * end-to-end number in bench.py. */
 size_t fa_host_arena_bytes(const fa_problem_t* p, int is_backward);
 int fa_forward_host(const fa_problem_t* p, const void* q, const void* k, const void* v,
                     void* o, void* l, void* m, void* dev_arena, size_t dev_arena_bytes, void* stream);

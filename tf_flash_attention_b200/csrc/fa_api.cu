@@ -65,6 +65,14 @@ bool is16(int dtype) { return dtype == FA_F16 || dtype == FA_BF16; }
 size_t elt(int dtype) { return is16(dtype) ? 2 : dtype == FA_F32 ? 4 : 8; }
 size_t l_elt(int dtype) { return dtype == FA_F64 ? 8 : 4; }
 
+// A workspace or host arena must be 256-byte aligned: the generic and fp64 kernels store double rows into the workspace
+// directly, and the tensor-core families carve TMA operands out of it.
+bool misaligned256(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 255) != 0; }
+bool bad_workspace(const void* ws, size_t bytes, size_t need) {
+  return bytes < need || (need && (!ws || misaligned256(ws)));
+}
+bool bad_arena(const void* arena, size_t bytes, size_t need) { return !arena || bytes < need || misaligned256(arena); }
+
 int cuda_fail(cudaError_t e) {
   fa::g_last_cuda = int(e);
   return FA_ECUDA;
@@ -107,7 +115,7 @@ const char* fa_strerror(int s) {
       return "stride size is too big; please make sure the stride size/window size is within the range "
              "representable by int32_t";
     case FA_EINVAL_SHAPE: return "invalid or unsupported shape";
-    case FA_EINVAL_WORKSPACE: return "workspace too small";
+    case FA_EINVAL_WORKSPACE: return "workspace (or host arena) too small, null or not 256-byte aligned";
     case FA_EINVAL_RANK: return "The number of dimensions of the inputs is inconsistent or too small";
     case FA_EINVAL_CHANNEL: return "The channel dimensions should be equal";
     case FA_EINVAL_BATCH: return "The batch shape of all inputs should be equal";
@@ -185,7 +193,7 @@ int fa_forward(const fa_problem_t* p, const void* q, const void* k, const void* 
   if (p->batch == 0) return FA_OK;
   if (!q || !k || !v || !o || !l || !m) return FA_EINVAL_NULL;
   const size_t need = fa_workspace_bytes(p, 0);
-  if (workspace_bytes < need || (!workspace && need)) return FA_EINVAL_WORKSPACE;
+  if (bad_workspace(workspace, workspace_bytes, need)) return FA_EINVAL_WORKSPACE;
   a.q = q; a.k = k; a.v = v; a.o = o; a.l = l; a.m = m;
   a.workspace = workspace; a.workspace_bytes = workspace_bytes;
   a.variant = fa::g_path_override;
@@ -218,7 +226,7 @@ int fa_backward(const fa_problem_t* p, const void* q, const void* k, const void*
   if (p->batch == 0) return FA_OK;
   if (!q || !k || !v || !o || !l || !m || !d_o || !d_q || !d_k || !d_v) return FA_EINVAL_NULL;
   const size_t need = fa_workspace_bytes(p, 1);
-  if (workspace_bytes < need || (!workspace && need)) return FA_EINVAL_WORKSPACE;
+  if (bad_workspace(workspace, workspace_bytes, need)) return FA_EINVAL_WORKSPACE;
   a.q = q; a.k = k; a.v = v; a.o = (void*)o; a.l = (void*)l; a.m = (void*)m; a.d_o = d_o;
   a.d_q = d_q; a.d_k = d_k; a.d_v = d_v;
   a.workspace = workspace; a.workspace_bytes = workspace_bytes;
@@ -279,7 +287,7 @@ int fa_backward_accumulate(const fa_problem_t* p, const void* q, const void* k, 
   if (p->batch == 0) return FA_OK;
   if (!q || !k || !v || !o || !l || !m || !d_o || !dq_acc || !d_k || !d_v) return FA_EINVAL_NULL;
   const size_t need = fa_workspace_bytes(p, 1);
-  if (workspace_bytes < need || (!workspace && need)) return FA_EINVAL_WORKSPACE;
+  if (bad_workspace(workspace, workspace_bytes, need)) return FA_EINVAL_WORKSPACE;
   if (!is16(p->dtype) || fa::g_path_override == 1 || !fa::sm100_f16_backward_accumulate_supports(a))
     return FA_EINVAL_SHAPE;   // callers fall back to fa_backward + fa_grad_accumulate
   fa::g_last_path = 2;
@@ -785,7 +793,7 @@ int fa_forward_host(const fa_problem_t* p, const void* q, const void* k, const v
   Arena a;
   int rc = arena_layout(p, 0, &a);
   if (rc) return rc;
-  if (!dev_arena || dev_arena_bytes < a.total) return FA_EINVAL_WORKSPACE;
+  if (bad_arena(dev_arena, dev_arena_bytes, a.total)) return FA_EINVAL_WORKSPACE;
   if (!q || !k || !v || !o || !l || !m) return FA_EINVAL_NULL;
   if (p->batch == 0) return FA_OK;
   char* base = (char*)dev_arena;
@@ -837,7 +845,7 @@ int backward_host_impl(const fa_problem_t* p, bool resident, const void* q, cons
   Arena a;
   int rc = arena_layout(p, 1, &a);
   if (rc) return rc;
-  if (!dev_arena || dev_arena_bytes < a.total) return FA_EINVAL_WORKSPACE;
+  if (bad_arena(dev_arena, dev_arena_bytes, a.total)) return FA_EINVAL_WORKSPACE;
   if (!resident && (!q || !k || !v || !o || !l || !m)) return FA_EINVAL_NULL;
   if (!d_o || !d_q || !d_k || !d_v) return FA_EINVAL_NULL;
   if (p->batch == 0) return FA_OK;
@@ -908,7 +916,7 @@ int fa_forward_backward_host(const fa_problem_t* p, const void* q, const void* k
   if (rc) return rc;
   if (p->accumulate) return FA_EINVAL_SHAPE;   // a step starts from fresh outputs
   const size_t need = fa_step_host_arena_bytes(p);
-  if (!dev_arena || dev_arena_bytes < need) return FA_EINVAL_WORKSPACE;
+  if (bad_arena(dev_arena, dev_arena_bytes, need)) return FA_EINVAL_WORKSPACE;
   if (!q || !k || !v || !d_o || !o || !l || !m || !d_q || !d_k || !d_v) return FA_EINVAL_NULL;
   if (p->batch == 0) return FA_OK;
   char* base = (char*)dev_arena;
